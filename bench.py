@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- BASELINE.json's headline metric on B200: batched ML-KEM-768 Encaps + Decaps.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--log2-items L] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--log2-items L] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3]): 2^22 synthetic ML-KEM-768 items PER GPU; one step = Encaps_internal over
 all items followed by Decaps_internal over the resulting ciphertexts with 10 % of them tampered (FO
@@ -44,6 +44,20 @@ UNIT = "encaps+decaps pairs/s"
 
 def emit(obj):
     print(json.dumps(obj), flush=True)
+
+
+# --dump-outputs: 8192 items x (1088 + 32 + 32) values as float32 = 37.7 MB per dump, whatever the batch size
+DUMP_ROWS = 8192
+
+
+def dump_rows(n: int):
+    """Indices (sorted) of the items whose outputs --dump-outputs writes: every item when n <= DUMP_ROWS, else a sample drawn
+    with a fixed seed, so that two builds run with the same arguments dump the same items."""
+    import numpy as np
+
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -116,7 +130,7 @@ def run_reference_arm(args):
         return
     threads = os.cpu_count() or 1
     # 32 pairs per thread and step: about 1.3 s per step at 20 ms per operation, whatever the core count
-    r = reference_pairs_per_s(threads, 32, max(1, args.steps), max(0, args.warmup))
+    r = reference_pairs_per_s(threads, 32, args.steps, max(0, args.warmup))
     emit({
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -197,8 +211,16 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--wc-inputs", action="store_true",
                     help="e2e input buffers in write-combined pinned memory where the box grants it (default: ordinary pinned memory)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm only (refused with --impl reference): write c, K (Encaps) and K' (Decaps) of the last timed step as "
+                         "float32 DIR/<name>.npy, rank 0's items (all of them up to %d, else a fixed seeded sample of that many: "
+                         "dump_rows)" % DUMP_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the GPU arm computed; it does not apply to --impl reference")
         return run_reference_arm(args)
 
     import numpy as np
@@ -294,6 +316,12 @@ def main():
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.summary(t_wall0, t_wall1)
     value = world * n * steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # here, before the legs below reuse c, K and Kd
+        rows = torch.from_numpy(dump_rows(n)).to(dev)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("encaps_c", c), ("encaps_K", K), ("decaps_K", Kd)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.index_select(0, rows).cpu().numpy().astype(np.float32))
 
     # ---- the two operations on their own (SURVEY 8(d): Encaps/s, Decaps/s and pairs/s = 1 / (1/E + 1/D)), device-resident, per GPU
     def timed_device(fn, reps=3):

@@ -53,3 +53,8 @@ def archive_stdout():
 @pytest.fixture(scope="session")
 def sha_examples():
     return json.load(open(os.path.join(GOLDEN, "sha_examples.json")))
+
+
+@pytest.fixture(scope="session")
+def reference_archive():
+    return json.load(open(os.path.join(GOLDEN, "reference_archive.json")))
