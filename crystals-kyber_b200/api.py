@@ -35,11 +35,66 @@ def _is_torch(x):
 class KeyTable:
     """Owner of a mlkem_b200_keys handle (freed, and wiped, with the object)."""
 
-    def __init__(self, kem, handle, ps):
-        self.kem, self.handle, self.ps = kem, handle, ps
+    def __init__(self, kem, handle, ps, device=-1):
+        self.kem, self.handle, self.ps, self.device = kem, handle, ps, device
 
     def __len__(self):
         return int(self.kem.lib.mlkem_b200_keys_count(self.handle))
+
+    def replace(self, slots, dk=None, ek=None, seeds=None, return_status=False):
+        """Overwrite the keys in `slots` in place with decapsulation keys `dk`, encapsulation keys `ek` (a table of
+        encapsulation keys only) or the 64-byte seeds `(d, z)` (KeyGen_internal on the device): mlkem_b200_keys_replace /
+        _replace_ek / _replace_from_seeds.  numpy key material goes through host memory, torch CUDA tensors through device memory
+        on the current torch stream; `slots` is always a host list.  return_status=True (dk only) also returns the dk hash
+        check per replaced key (0 / -5)."""
+        kem = self.kem
+        if _is_torch(slots):
+            slots = slots.cpu().numpy()
+        slots = np.ascontiguousarray(slots, np.uint32).ravel()
+        n = slots.size
+        prep = lambda a: a.contiguous() if _is_torch(a) else np.ascontiguousarray(a, np.uint8)
+        ptr = lambda a: C.c_void_p(a.data_ptr() if _is_torch(a) else a.ctypes.data)
+        sp = C.c_void_p(slots.ctypes.data)
+        status = None
+        if dk is not None:
+            dk = prep(dk)
+            o, _ = kem._src_opts(dk)
+            status = np.empty(n, np.int32) if return_status else None
+            rc = kem.lib.mlkem_b200_keys_replace(self.handle, n, sp, ptr(dk), None if status is None else C.c_void_p(status.ctypes.data),
+                                                 C.byref(o))
+            fname = "mlkem_b200_keys_replace"
+        elif ek is not None:
+            ek = prep(ek)
+            o, _ = kem._src_opts(ek)
+            rc = kem.lib.mlkem_b200_keys_replace_ek(self.handle, n, sp, ptr(ek), C.byref(o))
+            fname = "mlkem_b200_keys_replace_ek"
+        else:
+            d, z = (prep(a) for a in seeds)
+            o, _ = kem._src_opts(d, z)
+            rc = kem.lib.mlkem_b200_keys_replace_from_seeds(self.handle, n, sp, ptr(d), ptr(z), C.byref(o))
+            fname = "mlkem_b200_keys_replace_from_seeds"
+        kem._check(rc, fname)
+        return status if return_status else None
+
+    def export_ek(self, first=0, n=None, device=False):
+        """Encapsulation keys of rows [first, first + n) (default: to the end) -- mlkem_b200_keys_export_ek.  Returns numpy, or
+        with device=True a torch CUDA tensor on the table's device, filled on the current torch stream."""
+        kem = self.kem
+        ekb = sizes(self.ps)["ek"]
+        n = max(len(self) - first, 0) if n is None else n
+        if device:
+            import torch
+
+            dev = self.device if self.device >= 0 else torch.cuda.current_device()
+            out = torch.empty((n, ekb), dtype=torch.uint8, device=f"cuda:{dev}")
+            o = kem._opts(True, dev, torch.cuda.current_stream(dev).cuda_stream)
+            p = C.c_void_p(out.data_ptr())
+        else:
+            out = np.empty((n, ekb), np.uint8)
+            o = kem._opts(False)
+            p = C.c_void_p(out.ctypes.data)
+        kem._check(kem.lib.mlkem_b200_keys_export_ek(self.handle, first, n, p, C.byref(o)), "mlkem_b200_keys_export_ek")
+        return out
 
     def free(self):
         if self.handle:
@@ -189,7 +244,7 @@ class MLKEM:
             o.flags |= 4 if expand else 0
             rc = self.lib.mlkem_b200_keys_from_seeds(ps, self._count(d, 32), ptr(d), ptr(z), C.byref(o), C.byref(handle))
         self._check(rc, "mlkem_b200_keys_load")
-        table = KeyTable(self, handle, ps)
+        table = KeyTable(self, handle, ps, o.device)
         return (table, status) if return_status else table
 
     def _keyed(self, fname, table, key_index, data, item_bytes, out_shapes):

@@ -1364,6 +1364,143 @@ int keyed_opts(const mlkem_b200_keys *k, const mlkem_b200_opts *o, mlkem_b200_op
     return 0;
 }
 
+// ---- key rotation: rows of a live table replaced in place, ek rows read back ----------------------------------------
+// A replace or an export touches a table that keyed calls may still be reading, on any stream.  It needs no bookkeeping of
+// its own: every library call makes its stream wait for the slot events it uses and records them after its last kernel
+// (DeviceCtx::ev_slot), so a stream that waits for all kSlots of them, under call_mutex, is ordered after every call already
+// enqueued on the device, and recording them all afterwards orders every later call after it.
+int wait_all_slots(DeviceCtx *ctx, cudaStream_t st) {
+    for (int e = 0; e < kSlots; e++) CU(cudaStreamWaitEvent(st, ctx->ev_slot[e], 0));
+    return 0;
+}
+int record_all_slots(DeviceCtx *ctx, cudaStream_t st) {
+    for (int e = 0; e < kSlots; e++) CU(cudaEventRecord(ctx->ev_slot[e], st));
+    return 0;
+}
+
+// The slots of a replace are HOST memory: each < n_keys and none twice.  Checked before anything is written.
+int check_slots(const mlkem_b200_keys *k, size_t n, const uint32_t *slot) {
+    std::vector<uint32_t> s(slot, slot + n);
+    std::sort(s.begin(), s.end());
+    if (s.back() >= k->n) {
+        snprintf(tl_error, sizeof tl_error, "slot %u is outside the table of %zu keys", s.back(), k->n);
+        return MLKEM_B200_ERR_ARG;
+    }
+    auto dup = std::adjacent_find(s.begin(), s.end());
+    if (dup != s.end()) {
+        snprintf(tl_error, sizeof tl_error, "slot %u is listed twice", *dup);
+        return MLKEM_B200_ERR_ARG;
+    }
+    return 0;
+}
+
+// Device scratch that holds new key material (dk rows, seeds): wiped once its stream has drained, then freed.  Declared after
+// the DeviceGuard of the call, so that it is released on the call's device.
+struct WipedScratch {
+    void *p = nullptr;
+    size_t bytes = 0;
+    cudaStream_t st = nullptr;
+    ~WipedScratch() {
+        if (!p) return;
+        cudaStreamSynchronize(st);
+        cudaMemsetAsync(p, 0, bytes, st);
+        cudaStreamSynchronize(st);
+        cudaFree(p);
+    }
+};
+
+int scatter_rows(cudaStream_t st, size_t n, const uint8_t *src, size_t row_bytes, KeySel slots, uint8_t *dst) {
+    const size_t words = n * (row_bytes / 16);
+    LAUNCH(k_scatter_rows, std::min<unsigned>(cdiv(words, 256), 148 * 16), 256, 0, st, (int)n, (int)(row_bytes / 16), src, row_bytes, slots, dst,
+           row_bytes);
+    return 0;
+}
+
+enum class NewKeys { kDk, kEk, kSeeds };
+
+// mlkem_b200_keys_replace / _replace_ek / _replace_from_seeds.  `a` is dk, ek or d (then `z` is z).  The new rows, their H(ek),
+// the hash check and (expanded tables) their matrices are computed in device scratch on `st` first; only then does the stream
+// wait for the calls in flight and scatter the results into the listed rows of the table.
+int keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *a, const uint8_t *z, int32_t *status,
+                 const mlkem_b200_opts *o, NewKeys src) {
+    mlkem_b200_opts oo;
+    if (int rc = keyed_opts(k, o, &oo)) return rc;
+    const bool with_dk = src != NewKeys::kEk;
+    if (with_dk != (k->dk != nullptr)) {
+        snprintf(tl_error, sizeof tl_error, with_dk ? "the key table holds encapsulation keys only"
+                                                    : "the key table holds decapsulation keys: replace them, not their ek rows");
+        return MLKEM_B200_ERR_ARG;
+    }
+    if (n == 0) return MLKEM_B200_OK;
+    if (!slot || !a || (src == NewKeys::kSeeds && !z)) {
+        snprintf(tl_error, sizeof tl_error, "NULL buffer");
+        return MLKEM_B200_ERR_ARG;
+    }
+    if (int rc = check_slots(k, n, slot)) return rc;
+    const int set = k->set;
+    const unsigned kk = k_of(set), ekb = mlkem_b200_ek_bytes(set);
+    const size_t row = with_dk ? mlkem_b200_dk_bytes(set) : ekb, entries = k->matrix ? n * kk * kk : 0;
+    int dev;
+    DeviceCtx *ctx;
+    DeviceGuard guard;
+    if (int rc = acquire(&oo, &dev, &ctx, guard)) return rc;
+    const bool src_dev = oo.mem == MLKEM_B200_MEM_DEVICE;
+    // device-memory sources are read in order on the caller's stream
+    cudaStream_t st = src_dev ? static_cast<cudaStream_t>(oo.stream) : ctx->stream[0];
+    auto up = [](size_t b) { return (b + 255) & ~size_t(255); };
+    WipedScratch s;
+    s.st = st;
+    s.bytes = up(4 * n) + up(n * row) + up(32 * n) + up(4 * n) + (src == NewKeys::kSeeds ? up(64 * n) + up(n * ekb) : 0) +
+              (entries ? up(entries * 34 + 16) + up(entries * 512) : 0);
+    if (cudaMalloc(&s.p, s.bytes) != cudaSuccess) {
+        s.p = nullptr;
+        cudaGetLastError();
+        snprintf(tl_error, sizeof tl_error, "cudaMalloc of %zu bytes of replace scratch failed", s.bytes);
+        return MLKEM_B200_ERR_CUDA;
+    }
+    Arena ar(s.p);
+    uint32_t *d_slot = ar.take<uint32_t>(n);
+    uint8_t *rows = ar.take<uint8_t>(n * row), *hek = ar.take<uint8_t>(32 * n);
+    int32_t *d_status = ar.take<int32_t>(n);
+    const cudaMemcpyKind kind = src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    CU(cudaMemcpyAsync(d_slot, slot, 4 * n, cudaMemcpyHostToDevice, st));
+    if (src == NewKeys::kSeeds) {  // KeyGen_internal (ml_kem.c:1034) into scratch, as mlkem_b200_keys_from_seeds does
+        uint8_t *dz = ar.take<uint8_t>(64 * n), *ek_out = ar.take<uint8_t>(n * ekb);
+        CU(cudaMemcpyAsync(dz, a, 32 * n, kind, st));
+        CU(cudaMemcpyAsync(dz + 32 * n, z, 32 * n, kind, st));
+        mlkem_b200_opts od{dev, MLKEM_B200_MEM_DEVICE, st, 0, oo.sample_group_limit, oo.flags & MLKEM_B200_FLAG_FIPS203};
+        if (int rc = mlkem_b200_keygen_batch(set, n, dz, dz + 32 * n, ek_out, rows, &od)) return rc;
+    } else {
+        CU(cudaMemcpyAsync(rows, a, n * row, kind, st));
+    }
+    const uint8_t *ek_rows = with_dk ? rows + 384 * kk : rows;
+    DISPATCH_SET(set, LAUNCH((k_hash_ek_table<P>), cdiv(n, kHashTPB), kHashTPB, 0, st, (int)n, ek_rows, row, hek));
+    mlkem_b200_opts od{dev, MLKEM_B200_MEM_DEVICE, st, 0, 0, 0};
+    if (status && src == NewKeys::kDk)  // the hash check of KEM_Decaps (ml_kem.c:1336-1350) per new key, as in mlkem_b200_keys_load
+        if (int rc = mlkem_b200_check_dk_batch(set, n, rows, d_status, &od)) return rc;
+    uint16_t *mat = nullptr;
+    if (entries) {  // the matrices of the new keys, sampled with the group limit the table was loaded with
+        uint8_t *seeds = ar.take<uint8_t>(entries * 34 + 16);
+        mat = ar.take<uint16_t>(entries * 256);
+        DISPATCH_SET(set, LAUNCH((k_matrix_seeds<P>), cdiv(entries, 256), 256, 0, st, (int)n, ek_rows, row, seeds));
+        od.sample_group_limit = k->group_limit;
+        if (int rc = mlkem_b200_sample_ntt_batch(entries, seeds, mat, nullptr, &od)) return rc;
+    }
+    {
+        std::lock_guard<std::mutex> call_lock(ctx->call_mutex);
+        if (int rc = wait_all_slots(ctx, st)) return rc;
+        const KeySel sel{d_slot, 0, (uint32_t)k->n};
+        int rc = scatter_rows(st, n, rows, row, sel, with_dk ? k->dk : k->ek);
+        if (!rc) rc = scatter_rows(st, n, hek, 32, sel, k->hek);
+        if (!rc && mat) rc = scatter_rows(st, n, (const uint8_t *)mat, (size_t)kk * kk * 512, sel, (uint8_t *)k->matrix);
+        const int rc_rec = record_all_slots(ctx, st);  // also after a failed launch: the slots stay ordered
+        if (rc || rc_rec) return rc ? rc : rc_rec;
+    }
+    if (status && src == NewKeys::kDk) CU(cudaMemcpyAsync(status, d_status, 4 * n, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));  // a set-up call: the table is updated when it returns
+    return MLKEM_B200_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1432,6 +1569,52 @@ int mlkem_b200_keys_from_seeds(int set, size_t n_keys, const uint8_t *d, const u
 
 size_t mlkem_b200_keys_count(const mlkem_b200_keys *k) { return k ? k->n : 0; }
 void mlkem_b200_keys_free(mlkem_b200_keys *k) { keys_destroy(k); }
+
+int mlkem_b200_keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *dk, int32_t *status, const mlkem_b200_opts *o) {
+    return keys_replace(k, n, slot, dk, nullptr, status, o, NewKeys::kDk);
+}
+int mlkem_b200_keys_replace_ek(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *ek, const mlkem_b200_opts *o) {
+    return keys_replace(k, n, slot, ek, nullptr, nullptr, o, NewKeys::kEk);
+}
+int mlkem_b200_keys_replace_from_seeds(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *d, const uint8_t *z,
+                                       const mlkem_b200_opts *o) {
+    return keys_replace(k, n, slot, d, z, nullptr, o, NewKeys::kSeeds);
+}
+
+int mlkem_b200_keys_export_ek(const mlkem_b200_keys *k, size_t first, size_t n, uint8_t *ek, const mlkem_b200_opts *o) {
+    mlkem_b200_opts oo;
+    if (int rc = keyed_opts(k, o, &oo)) return rc;
+    if (first > k->n || n > k->n - first) {
+        snprintf(tl_error, sizeof tl_error, "rows [%zu, %zu + %zu) are outside the table of %zu keys", first, first, n, k->n);
+        return MLKEM_B200_ERR_ARG;
+    }
+    if (n == 0) return MLKEM_B200_OK;
+    if (!ek) {
+        snprintf(tl_error, sizeof tl_error, "NULL buffer");
+        return MLKEM_B200_ERR_ARG;
+    }
+    int dev;
+    DeviceCtx *ctx;
+    DeviceGuard guard;
+    if (int rc = acquire(&oo, &dev, &ctx, guard)) return rc;
+    const bool dst_dev = oo.mem == MLKEM_B200_MEM_DEVICE;
+    cudaStream_t st = dst_dev ? static_cast<cudaStream_t>(oo.stream) : ctx->stream[0];
+    const size_t ekb = mlkem_b200_ek_bytes(k->set);
+    {
+        std::lock_guard<std::mutex> call_lock(ctx->call_mutex);  // ordered like a replace (wait_all_slots)
+        if (int rc = wait_all_slots(ctx, st)) return rc;
+        const cudaError_t e = cudaMemcpy2DAsync(ek, ekb, k->ek + first * k->ek_stride, k->ek_stride, ekb, n,
+                                                dst_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st);
+        const int rc_rec = record_all_slots(ctx, st);
+        if (e != cudaSuccess) {
+            snprintf(tl_error, sizeof tl_error, "cudaMemcpy2DAsync failed: %s", cudaGetErrorString(e));
+            return MLKEM_B200_ERR_CUDA;
+        }
+        if (rc_rec) return rc_rec;
+    }
+    if (!dst_dev) CU(cudaStreamSynchronize(st));
+    return MLKEM_B200_OK;
+}
 
 int mlkem_b200_encaps_keyed_batch(const mlkem_b200_keys *k, size_t n, const uint32_t *key_index, const uint8_t *m, uint8_t *c, uint8_t *K,
                                   const mlkem_b200_opts *o) {

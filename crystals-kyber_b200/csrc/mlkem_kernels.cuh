@@ -1092,6 +1092,20 @@ __global__ void __launch_bounds__(256) k_matrix_seeds(int n, const uint8_t *__re
     out[33] = (uint8_t)col;
 }
 
+// Key rotation (mlkem_b200_keys_replace*): row i of src (src + i*src_stride) is copied to row key_row(slots, i) of dst,
+// 16 bytes per thread.  The new dk / ek rows, their H(ek) and their matrices are computed in scratch beforehand, so this is
+// the only kernel that writes into a live table, and it writes nothing outside the listed rows.  Strides and row sizes are
+// multiples of 16 (DK, EK, 384 K, 32, K*K*512).
+__global__ void __launch_bounds__(256) k_scatter_rows(int n, int row_words, const uint8_t *__restrict__ src, size_t src_stride, KeySel slots,
+                                                      uint8_t *__restrict__ dst, size_t dst_stride) {
+    const size_t total = (size_t)n * row_words;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const int i = (int)(t / row_words), w = (int)(t - (size_t)i * row_words);
+        const uint4 v = reinterpret_cast<const uint4 *>(src + src_stride * i)[w];
+        reinterpret_cast<uint4 *>(dst + dst_stride * key_row(slots, i))[w] = v;
+    }
+}
+
 // u rows of K-PKE.Encrypt from the table (ml_kem.c:854-896): persistent warps, warp = one (item, row); the K matrix
 // polynomials of the row come from HBM / L2 with coalesced 32-bit loads (a coefficient pair per lane and load), the
 // vector, noise codes and ciphertext row are fetched one row ahead like in the fused kernel.

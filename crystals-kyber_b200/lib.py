@@ -52,6 +52,10 @@ SIGNATURES = {
     "mlkem_b200_keys_from_seeds": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _PO, C.POINTER(C.c_void_p)]),
     "mlkem_b200_keys_count": (C.c_size_t, [C.c_void_p]),
     "mlkem_b200_keys_free": (None, [C.c_void_p]),
+    "mlkem_b200_keys_replace": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_keys_replace_ek": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _PO]),
+    "mlkem_b200_keys_replace_from_seeds": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _P8, _PO]),
+    "mlkem_b200_keys_export_ek": (C.c_int, [C.c_void_p, C.c_size_t, C.c_size_t, _P8, _PO]),
     "mlkem_b200_encaps_keyed_batch": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _P8, _P8, _PO]),
     "mlkem_b200_decaps_keyed_batch": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _P8, _PO]),
     "mlkem_b200_kem_keygen_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _PO]),

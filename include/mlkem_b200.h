@@ -153,6 +153,40 @@ int mlkem_b200_keys_from_seeds(int param_set, size_t n_keys, const uint8_t *d, c
 size_t mlkem_b200_keys_count(const mlkem_b200_keys *keys);
 void mlkem_b200_keys_free(mlkem_b200_keys *keys); /* wipes the decapsulation keys, then frees the table */
 
+/* Key rotation: overwrite the keys in slots slot[0..n) of an existing table, in place.  The table keeps its parameter set,
+ * device, size and memory: pointers that keyed calls already enqueued hold stay valid.
+ *   Results    afterwards keyed Encaps / Decaps on slot[i] give byte for byte what the unkeyed calls give with the new key i;
+ *              every other slot is unchanged.  In a table loaded with MLKEM_B200_FLAG_EXPAND_KEYS the matrices of the replaced
+ *              slots are re-expanded with the sample_group_limit the table was loaded with, not this call's.
+ *   Buffers    slot is always HOST memory (n x uint32).  The key material lives in opts->mem; device-memory sources are read
+ *              in order on opts->stream.  opts->device must be -1 or the table's.
+ *   Ordering   a set-up call: it returns once the table is updated.  It is ordered after every library call already enqueued
+ *              on the table's device (MLKEM_B200_FLAG_ASYNC host-memory calls and device-memory calls on any stream
+ *              included), and every call enqueued after it returns sees the new keys.
+ *   Errors     MLKEM_B200_ERR_ARG, with nothing written, for a slot >= n_keys, a slot listed twice, a NULL pointer, or the
+ *              wrong kind of table (see each function).  n == 0 does nothing and returns MLKEM_B200_OK.
+ *   Secrets    the old dk rows are overwritten in place; device scratch that held new dk bytes or seeds is zeroed before it
+ *              is freed. */
+/* New decapsulation keys: dk is n x (768k+96).  Not for a table of encapsulation keys only.  status (HOST memory, may be NULL)
+ * as in mlkem_b200_keys_load: status[i] = 0 or -5 from the dk hash check of key i (ml_kem.c:1336-1350); a failing key is
+ * written all the same. */
+int mlkem_b200_keys_replace(mlkem_b200_keys *keys, size_t n, const uint32_t *slot, const uint8_t *dk, int32_t *status,
+                            const mlkem_b200_opts *opts);
+/* New encapsulation keys: ek is n x (384k+32).  Only for a table of encapsulation keys (mlkem_b200_keys_load_ek): in a table
+ * with decapsulation keys the dk rows would contradict their ek. */
+int mlkem_b200_keys_replace_ek(mlkem_b200_keys *keys, size_t n, const uint32_t *slot, const uint8_t *ek,
+                               const mlkem_b200_opts *opts);
+/* The same as mlkem_b200_keys_replace with the dk of KeyGen_internal(d, z) (ml_kem.c:1034), run on the device: d, z are
+ * n x 32.  KeyGen honours opts->flags & MLKEM_B200_FLAG_FIPS203 and opts->sample_group_limit, as mlkem_b200_keys_from_seeds
+ * does.  Not for a table of encapsulation keys only. */
+int mlkem_b200_keys_replace_from_seeds(mlkem_b200_keys *keys, size_t n, const uint32_t *slot, const uint8_t *d,
+                                       const uint8_t *z, const mlkem_b200_opts *opts);
+/* Read back the encapsulation keys of rows [first, first + n) of a table (either kind) into ek (n x (384k+32), host or device
+ * memory per opts->mem): the public keys of a table built with mlkem_b200_keys_from_seeds, without a second KeyGen.  Ordered
+ * like a replace; a host-memory export returns when ek is filled, a device-memory one is enqueued on opts->stream.
+ * MLKEM_B200_ERR_ARG for a range outside the table or a NULL ek (n == 0: nothing to do, MLKEM_B200_OK). */
+int mlkem_b200_keys_export_ek(const mlkem_b200_keys *keys, size_t first, size_t n, uint8_t *ek, const mlkem_b200_opts *opts);
+
 /* Encaps_internal / Decaps_internal for n items, item i under key key_index[i] of the table.  key_index: n x uint32 in
  * the same memory space as the other buffers, or NULL = key (i mod n_keys).  Host-memory calls reject an index >=
  * n_keys (MLKEM_B200_ERR_ARG); device-memory calls clamp it to n_keys-1.  opts->device must be -1 or the table's. */
