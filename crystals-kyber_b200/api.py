@@ -32,6 +32,17 @@ def _is_torch(x):
     return type(x).__module__.startswith("torch")
 
 
+def _seed_ptr(seed):
+    """The call seed of the seeded calls as a host pointer: 32 bytes (bytes or a uint8 array), or None = fresh host entropy.
+    ctypes copies `bytes` into a buffer it owns for the duration of the call."""
+    if seed is None:
+        return None
+    b = bytes(np.ascontiguousarray(seed, np.uint8).ravel()) if not isinstance(seed, (bytes, bytearray)) else bytes(seed)
+    if len(b) != 32:
+        raise ValueError(f"the call seed is 32 bytes, got {len(b)}")
+    return C.c_char_p(b)
+
+
 class KeyTable:
     """Owner of a mlkem_b200_keys handle (freed, and wiped, with the object)."""
 
@@ -75,6 +86,17 @@ class KeyTable:
             fname = "mlkem_b200_keys_replace_from_seeds"
         kem._check(rc, fname)
         return status if return_status else None
+
+    def regenerate(self, slots, seed=None):
+        """Overwrite the keys in `slots` in place with KeyGen_internal(d_j, z_j) expanded on the device from the 32-byte call
+        seed (None: fresh host entropy) -- mlkem_b200_keys_replace_generate.  `slots` is a host list."""
+        kem = self.kem
+        if _is_torch(slots):
+            slots = slots.cpu().numpy()
+        slots = np.ascontiguousarray(slots, np.uint32).ravel()
+        o = kem._opts(False, self.device)
+        rc = kem.lib.mlkem_b200_keys_replace_generate(self.handle, slots.size, C.c_void_p(slots.ctypes.data), _seed_ptr(seed), C.byref(o))
+        kem._check(rc, "mlkem_b200_keys_replace_generate")
 
     def export_ek(self, first=0, n=None, device=False):
         """Encapsulation keys of rows [first, first + n) (default: to the end) -- mlkem_b200_keys_export_ek.  Returns numpy, or
@@ -304,6 +326,73 @@ class MLKEM:
                                                   C.c_void_p(c.ctypes.data), sz["c"] if c_len is None else c_len,
                                                   C.c_void_p(K.ctypes.data), C.c_void_p(status.ctypes.data), C.byref(o))
         return rc, K, status
+
+    # ------------------------------------------------------------------ randomness expanded on the device from a 32-byte call seed
+    # seed: 32 bytes (bytes or uint8 array) makes a call deterministic (tests, known answers); None draws it from the host entropy
+    # source.  Item j gets R_j = SHAKE256(seed || LE64(j) || LE64(tag)), see include/mlkem_b200.h.  Every call is synchronous.
+    def _out_opts(self, device_mem, shapes, dev=None):
+        """Empty outputs and options: numpy and host memory, or torch CUDA tensors on `dev` (default: the current device) and
+        device memory on its current torch stream."""
+        if device_mem:
+            import torch
+
+            dev = torch.cuda.current_device() if dev is None or dev < 0 else dev
+            outs = [torch.empty(s, dtype=torch.uint8, device=f"cuda:{dev}") for s in shapes]
+            return outs, self._opts(True, dev, torch.cuda.current_stream(dev).cuda_stream), lambda t: C.c_void_p(t.data_ptr())
+        return [np.empty(s, np.uint8) for s in shapes], self._opts(False, -1 if dev is None else dev), lambda a: C.c_void_p(a.ctypes.data)
+
+    def kem_keygen_seeded(self, ps, n, seed=None, device=False):
+        """KEM_KeyGen with (d_j, z_j) expanded on the GPU -- mlkem_b200_kem_keygen_seeded_batch.  Returns (ek, dk): numpy, or with
+        device=True torch CUDA tensors filled on the current torch stream."""
+        sz = sizes(ps if ps in PARAMS else 768)
+        (ek, dk), o, ptr = self._out_opts(device, [(n, sz["ek"]), (n, sz["dk"])])
+        rc = self.lib.mlkem_b200_kem_keygen_seeded_batch(ps, n, _seed_ptr(seed), ptr(ek), ptr(dk), C.byref(o))
+        self._check(rc, "mlkem_b200_kem_keygen_seeded_batch")
+        return ek, dk
+
+    def kem_encaps_seeded(self, ps, ek, seed=None, ek_len=None):
+        """KEM_Encaps with m_j expanded on the GPU -- mlkem_b200_kem_encaps_seeded_batch.  A numpy ek is host memory, a torch ek
+        device memory.  Returns (rc, c, K) like kem_encaps."""
+        sz = sizes(ps if ps in PARAMS else 768)  # an unknown set is the library's error to report (-1)
+        on_dev = _is_torch(ek)
+        if on_dev:
+            ek = ek.contiguous()
+            n = ek.numel() // sz["ek"] if ek_len is None else ek.shape[0]
+            (c, K), o, ptr = self._out_opts(True, [(n, sz["c"]), (n, 32)], ek.device.index)
+        else:
+            ek = np.ascontiguousarray(ek, np.uint8)
+            n = ek.size // sz["ek"] if ek_len is None else ek.shape[0]
+            (c, K), o, ptr = self._out_opts(False, [(n, sz["c"]), (n, 32)])
+        rc = self.lib.mlkem_b200_kem_encaps_seeded_batch(ps, n, ptr(ek), sz["ek"] if ek_len is None else ek_len, _seed_ptr(seed),
+                                                         ptr(c), ptr(K), C.byref(o))
+        return rc, c, K
+
+    def kem_encaps_keyed(self, table, n, key_index=None, seed=None, device=False):
+        """KEM_Encaps under table[key_index[i]] (None: key i mod n_keys) with m_j expanded on the GPU --
+        mlkem_b200_kem_encaps_keyed_batch.  Returns (c, K): numpy, or with device=True torch CUDA tensors on the table's device."""
+        (c, K), o, ptr = self._out_opts(device, [(n, sizes(table.ps)["c"]), (n, 32)], table.device)
+        idx = None
+        if key_index is not None:
+            if device:
+                import torch
+
+                idx = torch.as_tensor(key_index).to(device=c.device, dtype=torch.int32).contiguous()
+            else:
+                idx = np.ascontiguousarray(key_index.cpu().numpy() if _is_torch(key_index) else key_index, np.uint32)
+        rc = self.lib.mlkem_b200_kem_encaps_keyed_batch(table.handle, n, None if idx is None else ptr(idx), _seed_ptr(seed), ptr(c), ptr(K),
+                                                        C.byref(o))
+        self._check(rc, "mlkem_b200_kem_encaps_keyed_batch")
+        return c, K
+
+    def keys_generate(self, ps, n_keys, seed=None, device=None, expand=False):
+        """A resident key table of KeyGen_internal(d_j, z_j), j < n_keys, expanded on the GPU: its secrets never exist on the
+        host -- mlkem_b200_keys_generate.  Publish its keys with KeyTable.export_ek()."""
+        handle = C.c_void_p()
+        o = self._opts(False, -1 if device is None else device)
+        o.flags |= 4 if expand else 0
+        rc = self.lib.mlkem_b200_keys_generate(ps, n_keys, _seed_ptr(seed), C.byref(o), C.byref(handle))
+        self._check(rc, "mlkem_b200_keys_generate")
+        return KeyTable(self, handle, ps, o.device)
 
     # ------------------------------------------------------------------ K-PKE
     def pke_keygen(self, ps, d):

@@ -885,6 +885,92 @@ struct SyncOpts {
     }
 };
 
+// The modulus check of KEM_Encaps (ml_kem.c:1274-1291) for n keys: an identity in the reference (its ByteDecode12 never
+// reduces), see SURVEY D4.  In FIPS mode it is a real check: any coefficient >= q in any key rejects the call with -4.
+// Its MiscLease (device-memory calls) is released when it returns.
+static int fips_modulus_check(int set, size_t n, const uint8_t *ek, const mlkem_b200_opts *o) {
+    if (!fips_of(o)) return 0;
+    std::vector<int32_t> st_host(n);
+    const bool on_dev = o->mem == MLKEM_B200_MEM_DEVICE;
+    int dev;
+    DeviceCtx *ctx;
+    DeviceGuard guard;
+    MiscLease lease;
+    int32_t *status = st_host.data();
+    if (on_dev) {
+        if (int rc = acquire(o, &dev, &ctx, guard)) return rc;
+        if (int rc = lease.take(ctx, 4 * n, static_cast<cudaStream_t>(o->stream))) return rc;
+        status = reinterpret_cast<int32_t *>(lease.ptr);
+    }
+    int rc = MLKEM_B200_ERR_PARAM;
+    switch (set) {
+#define MODCHK(PS, PT)                                                                                                              \
+    case PS:                                                                                                                        \
+        rc = drive(o, n, 0, {{ek, nullptr, PT::EK}, {nullptr, status, 4}}, [=](cudaStream_t st, Arena &, int cn, void **p, size_t) { \
+            LAUNCH((k_check_ek_modulus<PT>), cdiv(cn, kHashTPB), kHashTPB, 0, st, cn, (const uint8_t *)p[0], (int *)p[1]);            \
+            return 0;                                                                                                               \
+        });                                                                                                                         \
+        break;
+        MODCHK(512, P512) MODCHK(768, P768) MODCHK(1024, P1024)
+#undef MODCHK
+    }
+    if (!rc && on_dev) {
+        cudaStream_t st = static_cast<cudaStream_t>(o->stream);
+        if (cudaMemcpyAsync(st_host.data(), status, 4 * n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            rc = MLKEM_B200_ERR_CUDA;
+    }
+    if (rc) return rc;
+    for (size_t i = 0; i < n; i++)
+        if (st_host[i] != 0) return MLKEM_B200_ERR_MODULUS;
+    return 0;
+}
+
+// ---- seeded randomness (include/mlkem_b200.h, "randomness expanded on the device") -------------------------------------
+// The 32-byte call seed of a seeded call: the caller's bytes, or 32 fresh bytes of host_entropy when seed is NULL.  It is
+// copied into the device's pooled misc scratch on `st`, ahead of every later use on that stream; the host copy is zeroed with
+// explicit_bzero and the device copy by the lease (after `st` has drained) when the object goes out of scope.  A seed decides
+// every secret of its call, so it never sits in a kernel-parameter buffer the library cannot wipe.
+struct CallSeed {
+    struct Host {
+        uint8_t b[32] = {};
+        ~Host() { explicit_bzero(b, sizeof b); }
+    } host;
+    MiscLease lease;  // declared after `host`: drained and wiped first
+    const uint8_t *dev = nullptr;
+    int take(DeviceCtx *ctx, const uint8_t *seed, cudaStream_t st) {
+        if (seed) memcpy(host.b, seed, sizeof host.b);
+        else if (int rc = host_entropy(host.b, sizeof host.b)) return rc;
+        if (int rc = lease.take(ctx, sizeof host.b, st)) return rc;
+        CU(cudaMemcpyAsync(lease.ptr, host.b, sizeof host.b, cudaMemcpyHostToDevice, st));
+        dev = lease.ptr;
+        return 0;
+    }
+};
+constexpr uint32_t kSeedTagKeyGen = 1, kSeedTagEncaps = 2;
+
+// R_j of items first .. first + n - 1 into out0 (and out1): see k_expand_seed.
+static int expand_seed(cudaStream_t st, int n, const uint8_t *seed, size_t first, uint32_t tag, uint8_t *out0, uint8_t *out1) {
+    LAUNCH(k_expand_seed, cdiv(n, kHashTPB), kHashTPB, 0, st, n, seed, (unsigned long long)first, tag, out0, out1);
+    return 0;
+}
+
+// Runs `call(seed_on_device)` for a seeded unkeyed / keyed call with synchronous options `o` (SyncOpts): the seed is placed on
+// the caller's stream (device memory) or on a library stream that is drained before the call's own streams read it (host memory).
+template <class F>
+static int with_call_seed(const mlkem_b200_opts *o, const uint8_t *seed, F call) {
+    int dev;
+    DeviceCtx *ctx;
+    DeviceGuard guard;
+    if (int rc = acquire(o, &dev, &ctx, guard)) return rc;
+    const bool on_dev = o && o->mem == MLKEM_B200_MEM_DEVICE;
+    cudaStream_t st = on_dev ? static_cast<cudaStream_t>(o->stream) : ctx->stream[0];
+    CallSeed cs;
+    if (int rc = cs.take(ctx, seed, st)) return rc;
+    if (!on_dev) CU(cudaStreamSynchronize(st));
+    return call(cs.dev);
+}
+
 extern "C" {
 
 int mlkem_b200_kem_keygen_batch(int set, size_t n, uint8_t *ek, uint8_t *dk, const mlkem_b200_opts *opts) {
@@ -904,41 +990,7 @@ int mlkem_b200_kem_encaps_batch(int set, size_t n, const uint8_t *ek, size_t ek_
     // modulus check (ml_kem.c:1274-1291): an identity in the reference (its ByteDecode12 never reduces), see SURVEY D4.
     // In FIPS mode it is a real check: any coefficient >= q in any key rejects the call with -4.
     if (n == 0) return MLKEM_B200_OK;
-    if (fips_of(o)) {
-        std::vector<int32_t> st_host(n);
-        const bool on_dev = o->mem == MLKEM_B200_MEM_DEVICE;
-        int dev;
-        DeviceCtx *ctx;
-        DeviceGuard guard;
-        MiscLease lease;
-        int32_t *status = st_host.data();
-        if (on_dev) {
-            if (int rc = acquire(o, &dev, &ctx, guard)) return rc;
-            if (int rc = lease.take(ctx, 4 * n, static_cast<cudaStream_t>(o->stream))) return rc;
-            status = reinterpret_cast<int32_t *>(lease.ptr);
-        }
-        int rc = MLKEM_B200_ERR_PARAM;
-        switch (set) {
-#define MODCHK(PS, PT)                                                                                                              \
-    case PS:                                                                                                                        \
-        rc = drive(o, n, 0, {{ek, nullptr, PT::EK}, {nullptr, status, 4}}, [=](cudaStream_t st, Arena &, int cn, void **p, size_t) { \
-            LAUNCH((k_check_ek_modulus<PT>), cdiv(cn, kHashTPB), kHashTPB, 0, st, cn, (const uint8_t *)p[0], (int *)p[1]);            \
-            return 0;                                                                                                               \
-        });                                                                                                                         \
-        break;
-            MODCHK(512, P512) MODCHK(768, P768) MODCHK(1024, P1024)
-#undef MODCHK
-        }
-        if (!rc && on_dev) {
-            cudaStream_t st = static_cast<cudaStream_t>(o->stream);
-            if (cudaMemcpyAsync(st_host.data(), status, 4 * n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess)
-                rc = MLKEM_B200_ERR_CUDA;
-        }
-        if (rc) return rc;
-        for (size_t i = 0; i < n; i++)
-            if (st_host[i] != 0) return MLKEM_B200_ERR_MODULUS;
-    }
+    if (int rc = fips_modulus_check(set, n, ek, o)) return rc;
     return with_entropy(o, 32 * n, [&](uint8_t *m) { return mlkem_b200_encaps_batch(set, n, ek, m, c, K, o); });
 }
 
@@ -965,6 +1017,49 @@ int mlkem_b200_kem_decaps_batch(int set, size_t n, const uint8_t *dk, size_t dk_
             if (status[i] != 0) memset(K + 32 * i, 0, 32);
     }
     return MLKEM_B200_OK;
+}
+
+// KEM_KeyGen with (d_j, z_j) expanded on the device from the call seed into the chunk workspace: nothing but the seed crosses
+// PCIe host-to-device.
+int mlkem_b200_kem_keygen_seeded_batch(int set, size_t n, const uint8_t *seed, uint8_t *ek, uint8_t *dk, const mlkem_b200_opts *opts) {
+    const SyncOpts so(opts);
+    const mlkem_b200_opts *o = so.p;
+    if (!mlkem_b200_ek_bytes(set)) return MLKEM_B200_ERR_PARAM;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(o);
+    const bool fips = fips_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        DISPATCH_SET(set, return drive(o, n, ws_bytes_per_item<P>() + 64, {{nullptr, ek, P::EK}, {nullptr, dk, P::DK}},
+                                       [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                                           uint8_t *d = ws.take<uint8_t>((size_t)cn * 32), *z = ws.take<uint8_t>((size_t)cn * 32);
+                                           if (int rc = expand_seed(st, cn, dseed, first, kSeedTagKeyGen, d, z)) return rc;
+                                           return enqueue_keygen<P>(st, ws, cn, d, z, (uint8_t *)p[0], (uint8_t *)p[1], gl, fips);
+                                       }));
+        return MLKEM_B200_ERR_PARAM;
+    });
+}
+
+// KEM_Encaps with m_j expanded on the device from the call seed: the checks of mlkem_b200_kem_encaps_batch, then Encaps_internal.
+int mlkem_b200_kem_encaps_seeded_batch(int set, size_t n, const uint8_t *ek, size_t ek_len, const uint8_t *seed, uint8_t *c, uint8_t *K,
+                                       const mlkem_b200_opts *opts) {
+    const SyncOpts so(opts);
+    const mlkem_b200_opts *o = so.p;
+    unsigned want = mlkem_b200_ek_bytes(set);
+    if (!want) return MLKEM_B200_ERR_PARAM;
+    if (ek_len != want) return MLKEM_B200_ERR_LENGTH;  // type check, ml_kem.c:1267
+    if (n == 0) return MLKEM_B200_OK;
+    if (int rc = fips_modulus_check(set, n, ek, o)) return rc;  // its lease is released before the seed's is taken
+    const int gl = group_limit_of(o);
+    const bool fips = fips_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        DISPATCH_SET(set, return drive(o, n, ws_bytes_per_item<P>() + 32, {{ek, nullptr, P::EK}, {nullptr, c, P::C}, {nullptr, K, 32}},
+                                       [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                                           uint8_t *m = ws.take<uint8_t>((size_t)cn * 32);
+                                           if (int rc = expand_seed(st, cn, dseed, first, kSeedTagEncaps, m, nullptr)) return rc;
+                                           return enqueue_encaps<P>(st, ws, cn, (const uint8_t *)p[0], m, (uint8_t *)p[1], (uint8_t *)p[2], gl, fips);
+                                       }));
+        return MLKEM_B200_ERR_PARAM;
+    });
 }
 
 int mlkem_b200_pke_encrypt_batch(int set, size_t n, const uint8_t *ek, const uint8_t *m, const uint8_t *r, uint8_t *c, const mlkem_b200_opts *o) {
@@ -1340,6 +1435,24 @@ int keys_create(int set, size_t n, bool with_dk, const mlkem_b200_opts *o, mlkem
     return MLKEM_B200_OK;
 }
 
+// The fill of mlkem_b200_keys_from_seeds / _keys_generate: KeyGen_internal (ml_kem.c:1034) into the table's dk rows from the
+// (d, z) that `place(dd, dz)` enqueues on `st` into a temporary, which is zeroed before it is freed.  A scratch ek array in the
+// same temporary receives KeyGen's first output (dk embeds the same bytes).
+template <class Place>
+int keygen_into_table(size_t n_keys, const mlkem_b200_opts *o, cudaStream_t st, mlkem_b200_keys *k, Place place) {
+    const unsigned ekb = mlkem_b200_ek_bytes(k->set);
+    uint8_t *tmp = nullptr;
+    CU(cudaMalloc(&tmp, n_keys * (ekb + 64)));
+    uint8_t *dd = tmp + n_keys * ekb, *dz = dd + 32 * n_keys;
+    int rc = place(dd, dz);
+    mlkem_b200_opts od{k->device, MLKEM_B200_MEM_DEVICE, st, 0, o ? o->sample_group_limit : 0, o ? o->flags : 0};
+    if (!rc) rc = mlkem_b200_keygen_batch(k->set, n_keys, dd, dz, tmp, k->dk, &od);
+    cudaStreamSynchronize(st);
+    cudaMemset(tmp, 0, n_keys * (ekb + 64));
+    cudaFree(tmp);
+    return rc;
+}
+
 // key_index of a keyed host-memory call is checked on the host; device-memory calls clamp in the kernel (key_row).
 int check_key_index(const mlkem_b200_keys *k, size_t n, const uint32_t *idx, const mlkem_b200_opts *o) {
     if (!idx || (o && o->mem == MLKEM_B200_MEM_DEVICE)) return 0;
@@ -1416,9 +1529,10 @@ int scatter_rows(cudaStream_t st, size_t n, const uint8_t *src, size_t row_bytes
     return 0;
 }
 
-enum class NewKeys { kDk, kEk, kSeeds };
+enum class NewKeys { kDk, kEk, kSeeds, kGenerate };
 
-// mlkem_b200_keys_replace / _replace_ek / _replace_from_seeds.  `a` is dk, ek or d (then `z` is z).  The new rows, their H(ek),
+// mlkem_b200_keys_replace / _replace_ek / _replace_from_seeds / _replace_generate.  `a` is dk, ek, d (then `z` is z) or the call
+// seed (may be NULL: fresh host entropy).  The new rows, their H(ek),
 // the hash check and (expanded tables) their matrices are computed in device scratch on `st` first; only then does the stream
 // wait for the calls in flight and scatter the results into the listed rows of the table.
 int keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *a, const uint8_t *z, int32_t *status,
@@ -1432,7 +1546,7 @@ int keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8
         return MLKEM_B200_ERR_ARG;
     }
     if (n == 0) return MLKEM_B200_OK;
-    if (!slot || !a || (src == NewKeys::kSeeds && !z)) {
+    if (!slot || (!a && src != NewKeys::kGenerate) || (src == NewKeys::kSeeds && !z)) {
         snprintf(tl_error, sizeof tl_error, "NULL buffer");
         return MLKEM_B200_ERR_ARG;
     }
@@ -1450,7 +1564,8 @@ int keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8
     auto up = [](size_t b) { return (b + 255) & ~size_t(255); };
     WipedScratch s;
     s.st = st;
-    s.bytes = up(4 * n) + up(n * row) + up(32 * n) + up(4 * n) + (src == NewKeys::kSeeds ? up(64 * n) + up(n * ekb) : 0) +
+    const bool keygen = src == NewKeys::kSeeds || src == NewKeys::kGenerate;
+    s.bytes = up(4 * n) + up(n * row) + up(32 * n) + up(4 * n) + (keygen ? up(64 * n) + up(n * ekb) : 0) +
               (entries ? up(entries * 34 + 16) + up(entries * 512) : 0);
     if (cudaMalloc(&s.p, s.bytes) != cudaSuccess) {
         s.p = nullptr;
@@ -1464,10 +1579,16 @@ int keys_replace(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8
     int32_t *d_status = ar.take<int32_t>(n);
     const cudaMemcpyKind kind = src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     CU(cudaMemcpyAsync(d_slot, slot, 4 * n, cudaMemcpyHostToDevice, st));
-    if (src == NewKeys::kSeeds) {  // KeyGen_internal (ml_kem.c:1034) into scratch, as mlkem_b200_keys_from_seeds does
+    if (keygen) {  // KeyGen_internal (ml_kem.c:1034) into scratch, as mlkem_b200_keys_from_seeds does
         uint8_t *dz = ar.take<uint8_t>(64 * n), *ek_out = ar.take<uint8_t>(n * ekb);
-        CU(cudaMemcpyAsync(dz, a, 32 * n, kind, st));
-        CU(cudaMemcpyAsync(dz + 32 * n, z, 32 * n, kind, st));
+        if (src == NewKeys::kSeeds) {
+            CU(cudaMemcpyAsync(dz, a, 32 * n, kind, st));
+            CU(cudaMemcpyAsync(dz + 32 * n, z, 32 * n, kind, st));
+        } else {  // (d_j, z_j) of the j-th listed slot, expanded from the call seed; its lease ends here, before call_mutex is taken
+            CallSeed cs;
+            if (int rc = cs.take(ctx, a, st)) return rc;
+            if (int rc = expand_seed(st, (int)n, cs.dev, 0, kSeedTagKeyGen, dz, dz + 32 * n)) return rc;
+        }
         mlkem_b200_opts od{dev, MLKEM_B200_MEM_DEVICE, st, 0, oo.sample_group_limit, oo.flags & MLKEM_B200_FLAG_FIPS203};
         if (int rc = mlkem_b200_keygen_batch(set, n, dz, dz + 32 * n, ek_out, rows, &od)) return rc;
     } else {
@@ -1546,24 +1667,58 @@ int mlkem_b200_keys_load_ek(int set, size_t n_keys, const uint8_t *ek, const mlk
 
 int mlkem_b200_keys_from_seeds(int set, size_t n_keys, const uint8_t *d, const uint8_t *z, const mlkem_b200_opts *o, mlkem_b200_keys **out) {
     if (!d || !z) return MLKEM_B200_ERR_ARG;
-    const unsigned ekb = mlkem_b200_ek_bytes(set);
     const bool src_dev = o && o->mem == MLKEM_B200_MEM_DEVICE;
     // KeyGen_internal on the device (ml_kem.c:1034): 64 bytes per key cross PCIe instead of 2400, and KeyGen is faster than
-    // the copy it replaces.  A scratch ek array receives KeyGen's first output (dk embeds the same bytes).
+    // the copy it replaces.
     return keys_create(set, n_keys, true, o, out, [&](DeviceCtx *, cudaStream_t st, mlkem_b200_keys *k) -> int {
-        uint8_t *tmp = nullptr;
-        CU(cudaMalloc(&tmp, n_keys * (ekb + 64)));
-        uint8_t *dd = tmp + n_keys * ekb, *dz = dd + 32 * n_keys;
-        const cudaMemcpyKind kind = src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-        int rc = 0;
-        if (cudaMemcpyAsync(dd, d, 32 * n_keys, kind, st) != cudaSuccess || cudaMemcpyAsync(dz, z, 32 * n_keys, kind, st) != cudaSuccess)
-            rc = MLKEM_B200_ERR_CUDA;
-        mlkem_b200_opts od{k->device, MLKEM_B200_MEM_DEVICE, st, 0, o ? o->sample_group_limit : 0, o ? o->flags : 0};
-        if (!rc) rc = mlkem_b200_keygen_batch(set, n_keys, dd, dz, tmp, k->dk, &od);
-        cudaStreamSynchronize(st);
-        cudaMemset(tmp, 0, n_keys * (ekb + 64));
-        cudaFree(tmp);
-        return rc;
+        return keygen_into_table(n_keys, o, st, k, [&](uint8_t *dd, uint8_t *dz) -> int {
+            const cudaMemcpyKind kind = src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+            CU(cudaMemcpyAsync(dd, d, 32 * n_keys, kind, st));
+            CU(cudaMemcpyAsync(dz, z, 32 * n_keys, kind, st));
+            return 0;
+        });
+    });
+}
+
+// mlkem_b200_keys_from_seeds with (d_j, z_j) expanded on the device from the call seed: the secrets of the table never exist on
+// the host.
+int mlkem_b200_keys_generate(int set, size_t n_keys, const uint8_t *seed, const mlkem_b200_opts *opts, mlkem_b200_keys **out) {
+    const SyncOpts so(opts);
+    const mlkem_b200_opts *o = so.p;
+    return keys_create(set, n_keys, true, o, out, [&](DeviceCtx *ctx, cudaStream_t st, mlkem_b200_keys *k) -> int {
+        return keygen_into_table(n_keys, o, st, k, [&](uint8_t *dd, uint8_t *dz) -> int {
+            CallSeed cs;  // one lease at a time: this one ends (device copy wiped) before KeyGen runs
+            if (int rc = cs.take(ctx, seed, st)) return rc;
+            return expand_seed(st, (int)n_keys, cs.dev, 0, kSeedTagKeyGen, dd, dz);
+        });
+    });
+}
+
+int mlkem_b200_keys_replace_generate(mlkem_b200_keys *k, size_t n, const uint32_t *slot, const uint8_t *seed, const mlkem_b200_opts *o) {
+    return keys_replace(k, n, slot, seed, nullptr, nullptr, o, NewKeys::kGenerate);
+}
+
+int mlkem_b200_kem_encaps_keyed_batch(const mlkem_b200_keys *k, size_t n, const uint32_t *key_index, const uint8_t *seed, uint8_t *c, uint8_t *K,
+                                      const mlkem_b200_opts *opts) {
+    const SyncOpts so(opts);
+    mlkem_b200_opts oo;
+    if (int rc = keyed_opts(k, so.p, &oo)) return rc;
+    if (int rc = check_key_index(k, n, key_index, &oo)) return rc;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(&oo);
+    const bool fips = fips_of(&oo), has_idx = key_index != nullptr;
+    const uint32_t nk = (uint32_t)k->n;
+    std::vector<Buf> bufs = {{nullptr, c, mlkem_b200_ct_bytes(k->set)}, {nullptr, K, 32}};
+    if (has_idx) bufs.push_back({key_index, nullptr, 4});
+    return with_call_seed(&oo, seed, [&](const uint8_t *dseed) -> int {
+        DISPATCH_SET(k->set, return drive(&oo, n, ws_bytes_per_item<P>() + 32, bufs, [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                         uint8_t *m = ws.take<uint8_t>((size_t)cn * 32);
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagEncaps, m, nullptr)) return rc;
+                         KeySel ks{has_idx ? (const uint32_t *)p[2] : nullptr, (uint32_t)(first % nk), nk};
+                         return enqueue_encaps_keyed<P>(st, ws, cn, k->ek, k->ek_stride, k->hek, ks, m, (uint8_t *)p[0], (uint8_t *)p[1], gl, fips,
+                                                        k->matrix);
+                     }));
+        return MLKEM_B200_ERR_PARAM;
     });
 }
 

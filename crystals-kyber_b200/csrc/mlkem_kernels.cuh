@@ -1106,6 +1106,29 @@ __global__ void __launch_bounds__(256) k_scatter_rows(int n, int row_words, cons
     }
 }
 
+// Randomness of the seeded calls (mlkem_b200_kem_*_seeded_batch, _kem_encaps_keyed_batch, _keys_generate, _keys_replace_generate):
+// R_j = SHAKE256(seed[32] || LE64(first + j) || LE64(tag)), 48 bytes = 6 lanes, one block at rate 136, one permutation.  R_j[0:32]
+// goes to out0 + 32 j (d of KeyGen, m of Encaps) and, when out1 is not null, R_j[32:64] to out1 + 32 j (z of KeyGen): the two
+// arrays enqueue_keygen takes.  `first` is the index within the whole call of this launch's first item, so the result does not
+// depend on the chunking.  The 32-byte call seed is read from device memory, never passed as a kernel argument.
+__global__ void __launch_bounds__(kHashTPB) k_expand_seed(int n, const uint8_t *__restrict__ seed, unsigned long long first, uint32_t tag,
+                                                          uint8_t *__restrict__ out0, uint8_t *__restrict__ out1) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const unsigned long long idx = first + (unsigned long long)j;
+    Lane a[25];
+    sponge_absorb_words<kRateSha3_256>(a, 6, kSfxXof, [&](int w) {
+        if (w < 4) return load_lane(seed + 8 * w);
+        return w == 4 ? Lane{(uint32_t)idx, (uint32_t)(idx >> 32)} : Lane{tag, 0u};
+    });
+#pragma unroll
+    for (int w = 0; w < 4; w++) store_lane(out0 + 32 * (size_t)j + 8 * w, a[w]);
+    if (out1) {
+#pragma unroll
+        for (int w = 0; w < 4; w++) store_lane(out1 + 32 * (size_t)j + 8 * w, a[4 + w]);
+    }
+}
+
 // u rows of K-PKE.Encrypt from the table (ml_kem.c:854-896): persistent warps, warp = one (item, row); the K matrix
 // polynomials of the row come from HBM / L2 with coalesced 32-bit loads (a coefficient pair per lane and load), the
 // vector, noise codes and ciphertext row are fetched one row ahead like in the fused kernel.

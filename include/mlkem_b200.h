@@ -226,6 +226,55 @@ int mlkem_b200_kem_encaps_batch(int param_set, size_t n, const uint8_t *ek, size
 int mlkem_b200_kem_decaps_batch(int param_set, size_t n, const uint8_t *dk, size_t dk_len, const uint8_t *c, size_t c_len,
                                 uint8_t *K, int32_t *status, const mlkem_b200_opts *opts);
 
+/* ---- randomness expanded on the device: KEM_KeyGen / KEM_Encaps, keyed KEM_Encaps, generated key tables -------------- */
+
+/* The calls above read every random byte from /dev/urandom on one host thread (64 bytes per KeyGen, 32 per Encaps), far
+ * below what the device computes.  The calls below take ONE 32-byte call seed and expand it on the device.  Item j of a call
+ * (its position in the call, 0 <= j < n, whatever the chunking) gets
+ *
+ *     R_j = SHAKE256(seed[0..32) || LE64(j) || LE64(tag), 64 bytes)    -- 48 input bytes: one block, one Keccak-f[1600]
+ *
+ *   tag 1 (KeyGen):  d_j = R_j[0..32), z_j = R_j[32..64)
+ *   tag 2 (Encaps):  m_j = R_j[0..32)
+ *
+ * and the call returns exactly what the named existing call returns with that randomness.
+ *
+ *   seed     always HOST memory, 32 bytes, or NULL.  NULL: 32 fresh bytes from the host entropy source (/dev/urandom) for this
+ *            call; -2 when that source fails, as in mlkem_b200_kem_keygen_batch.  A non-NULL seed makes the call deterministic:
+ *            that form is for tests and known-answer checks, like the *_internal calls.  A repeated seed repeats EVERY secret
+ *            of the call (every d, z, m and so every dk and shared key): never pass one twice outside a test.
+ *   Not a DRBG  this is a SHAKE256 expansion of 32 OS bytes per call, not an SP 800-90A DRBG.  Callers that need every random
+ *            byte from the OS keep mlkem_b200_kem_keygen_batch / _kem_encaps_batch.
+ *   Flags    the derivation does not depend on MLKEM_B200_FLAG_FIPS203; the KEM computations honour it as usual.
+ *   Secrets  the seed is copied into the device's pooled scratch; the library's host copy is zeroed with explicit_bzero and the
+ *            device copy once the call's work has drained, before the call returns: it never sits in a kernel-parameter
+ *            buffer.  The expanded d, z, m live only in the chunk workspaces or in scratch that is zeroed, like every other
+ *            per-item secret, and host-memory calls never send them over PCIe (a seeded KeyGen copies nothing to the device
+ *            but the seed).
+ *   Synchrony  so every call here is SYNCHRONOUS in both memory spaces: a device-memory call returns once opts->stream has
+ *            drained, and MLKEM_B200_FLAG_ASYNC is ignored.
+ * The other buffers follow opts->mem. */
+
+/* mlkem_b200_keygen_batch(d_j, z_j).  ek: n x (384k+32), dk: n x (768k+96). */
+int mlkem_b200_kem_keygen_seeded_batch(int param_set, size_t n, const uint8_t *seed, uint8_t *ek, uint8_t *dk,
+                                       const mlkem_b200_opts *opts);
+/* The checks of mlkem_b200_kem_encaps_batch (-1 unknown set, -3 ek_len, in FIPS mode -4 when any coefficient of any ek is
+ * >= q), then mlkem_b200_encaps_batch(ek, m_j). */
+int mlkem_b200_kem_encaps_seeded_batch(int param_set, size_t n, const uint8_t *ek, size_t ek_len, const uint8_t *seed,
+                                       uint8_t *c, uint8_t *K, const mlkem_b200_opts *opts);
+/* mlkem_b200_encaps_keyed_batch(keys, key_index, m_j), with its index rules (host memory rejects an index >= n_keys, device
+ * memory clamps it, NULL = i mod n_keys), on a table of either kind. */
+int mlkem_b200_kem_encaps_keyed_batch(const mlkem_b200_keys *keys, size_t n, const uint32_t *key_index, const uint8_t *seed,
+                                      uint8_t *c, uint8_t *K, const mlkem_b200_opts *opts);
+/* mlkem_b200_keys_from_seeds(d_j, z_j) for j < n_keys: a key table whose secrets never exist on the host.  Honours
+ * MLKEM_B200_FLAG_EXPAND_KEYS, MLKEM_B200_FLAG_FIPS203 and sample_group_limit.  Publish its keys with mlkem_b200_keys_export_ek. */
+int mlkem_b200_keys_generate(int param_set, size_t n_keys, const uint8_t *seed, const mlkem_b200_opts *opts,
+                             mlkem_b200_keys **out);
+/* mlkem_b200_keys_replace_from_seeds(slot, d_j, z_j), j the position in slot[]: the checks, ordering and errors of the other
+ * replaces. */
+int mlkem_b200_keys_replace_generate(mlkem_b200_keys *keys, size_t n, const uint32_t *slot, const uint8_t *seed,
+                                     const mlkem_b200_opts *opts);
+
 /* ---- K-PKE (FIPS 203 Alg. 13-15) -------------------------------------------------------------------- */
 
 /* PKE_KeyGen, ml_kem.c:651.  d: n x 32.  ek: n x (384k+32).  dk_pke: n x 384k. */
