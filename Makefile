@@ -1,6 +1,7 @@
 # Top-level build: the product library (CUDA, sm_100a), the INT32 microbenchmark and the checkers.
 #   make            -> crystals-kyber_b200/libmlkem_b200.so + build/microbench + oracle/
 #   make lib        -> only the product library
+#   make contracts  -> build/libmlkem_b200_contracts.so, the test-only harness of the device functions (tests/csrc/)
 NVCC    ?= /usr/local/cuda/bin/nvcc
 ARCH    := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS := $(ARCH) -O3 -std=c++17 -lineinfo -Xcompiler -fPIC,-fvisibility=hidden -cudart static
@@ -8,12 +9,18 @@ PKG     := crystals-kyber_b200
 CSRC    := $(PKG)/csrc
 LIB     := $(PKG)/libmlkem_b200.so
 
-all: lib tools examples oracle
+all: lib contracts tools examples oracle
 
 lib: $(LIB)
 
-$(LIB): $(CSRC)/mlkem_b200.cu $(CSRC)/mlkem_kernels.cuh $(CSRC)/mlkem_device.cuh $(CSRC)/ml_kem_compat.inl $(CSRC)/mlkem_profile.inl $(CSRC)/sha3_compat.inl include/mlkem_b200.h include/ml_kem.h include/sha3.h
+$(LIB): $(CSRC)/mlkem_b200.cu $(CSRC)/mlkem_kernels.cuh $(CSRC)/mlkem_device.cuh $(CSRC)/ml_kem_compat.inl $(CSRC)/mlkem_profile.inl $(CSRC)/sha3_compat.inl $(CSRC)/mlkem_tables.inl include/mlkem_b200.h include/ml_kem.h include/sha3.h
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(CSRC)/mlkem_b200.cu
+
+# test-only harness: the device functions of mlkem_device.cuh one by one, on the library's tables (tests/test_device_contracts_gpu.py)
+contracts: build/libmlkem_b200_contracts.so
+build/libmlkem_b200_contracts.so: tests/csrc/device_contracts.cu $(CSRC)/mlkem_device.cuh $(CSRC)/mlkem_tables.inl
+	mkdir -p build
+	$(NVCC) $(NVFLAGS) -shared -o $@ tests/csrc/device_contracts.cu
 
 # experiment build of the library (timing experiments that break the results on purpose: tools/time_encaps.py)
 exp: build/libmlkem_b200_exp.so
@@ -46,7 +53,7 @@ oracle: lib
 	$(MAKE) -C oracle drivers
 
 clean:
-	rm -f $(LIB) build/microbench build/keccak_bench build/coissue_bench
+	rm -f $(LIB) build/libmlkem_b200_contracts.so build/microbench build/keccak_bench build/coissue_bench
 	$(MAKE) -C oracle clean
 
-.PHONY: all lib exp tools examples oracle clean
+.PHONY: all lib contracts exp tools examples oracle clean

@@ -105,43 +105,7 @@ inline unsigned warp_grid(size_t items, int warps_per_block) {
 // ------------------------------------------------------------------------------------------------
 // Tables
 // ------------------------------------------------------------------------------------------------
-unsigned bitrev7(unsigned r) {
-    unsigned o = 0;
-    for (int i = 0; i < 7; i++) o |= ((r >> i) & 1u) << (6 - i);
-    return o;
-}
-unsigned pow17(unsigned e) {
-    unsigned z = 1;
-    while (e--) z = (z * 17u) % kQ;
-    return z;
-}
-uint2 shoup_pair(unsigned w) { return make_uint2(w, (w << 16) / kQ); }
-uint2 shoup_pair32(unsigned w) { return make_uint2(w, (unsigned)(((unsigned long long)w << 32) / kQ)); }
-
-void build_tables(TwiddleTables &t, uint2 rc[24]) {
-    for (unsigned i = 0; i < 128; i++) {
-        t.zeta[i] = shoup_pair(pow17(bitrev7(i)));           // ml_kem.c:300-307
-        t.gamma[i] = shoup_pair(pow17(2 * bitrev7(i) + 1));  // ml_kem.c:424-433
-        t.gamma32[i] = shoup_pair32(t.gamma[i].x);
-        t.zeta32[i] = shoup_pair32(t.zeta[i].x);
-    }
-    t.zeta_inv_last[0] = shoup_pair((t.zeta[1].x * 3303u) % kQ);  // ml_kem.c:378-381 folded into the last layer
-    t.zeta_inv_last[1] = shoup_pair(3303u);
-    t.zeta_inv_last32[0] = shoup_pair32(t.zeta_inv_last[0].x);
-    t.zeta_inv_last32[1] = shoup_pair32(3303u);
-    // Keccak round constants from the LFSR of FIPS 202 Alg. 5 (what sha3.c:148-205 recomputes every round)
-    uint8_t lfsr = 1;
-    for (int round = 0; round < 24; round++) {
-        unsigned long long c = 0;
-        for (int j = 0; j <= 6; j++) {
-            if (lfsr & 1) c |= 1ULL << ((1u << j) - 1);
-            uint8_t hi = lfsr & 0x80;
-            lfsr = (uint8_t)(lfsr << 1);
-            if (hi) lfsr ^= 0x71;
-        }
-        rc[round] = make_uint2((unsigned)c, (unsigned)(c >> 32));
-    }
-}
+#include "mlkem_tables.inl"
 
 // ------------------------------------------------------------------------------------------------
 // Per-device context

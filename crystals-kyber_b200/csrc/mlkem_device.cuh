@@ -96,7 +96,8 @@ __device__ __forceinline__ uint32_t mulz(uint32_t a, uint2 z) {  // z from the z
 // x mod q, exact, for x < 2^21 (1290168 = ceil(2^32 / q); checked exhaustively in
 // tests/test_abi_cpu.py::test_arithmetic_lemmas): two fma-pipe instructions, none on the alu pipe.
 __device__ __forceinline__ uint32_t canon_fma(uint32_t x) { return x - mulhi(x, 1290168u) * kQ; }
-// x mod q for x < 2^16, result in [0, q].
+// x mod q for x < 2^16, result in [0, q + 1]: q + 1 only for x = 56594, 59923, 63252, so the result is <= q for x < 16q
+// (checked exhaustively in tests/test_abi_cpu.py::test_arithmetic_lemmas).
 __device__ __forceinline__ uint32_t barrett16(uint32_t x) {
     uint32_t qh = (x * 40317u) >> 27;  // floor(2^27 / q) = 40317
     return x - qh * kQ;

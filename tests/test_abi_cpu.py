@@ -174,9 +174,27 @@ def test_arithmetic_lemmas():
     wy = (zetas << np.uint64(16)) // u(q)
     r = bb * zetas - ((bb * wy) >> np.uint64(16)) * u(q)
     assert (r < 2 * q).all() and (np.where(r >= q, r - u(q), r) == bb * zetas % u(q)).all()
-    xs = np.arange(4096 + q, dtype=np.uint64)
-    b16 = xs - ((xs * u(40317)) >> np.uint64(27)) * u(q)  # barrett16: result in [0, q]
-    assert (b16 <= q).all() and (np.where(b16 >= q, b16 - u(q), b16) == xs % u(q)).all()
+    # barrett16 (32-bit product, shift 27) on every x < 2^16: congruent, in [0, q + 1]; q + 1 at exactly three inputs, all
+    # above 16q = 53264, the bound of the sums that the balanced inverse transform reduces with barrett16 alone
+    barrett16 = lambda x: x - (((x * u(40317)) & u(0xFFFFFFFF)) >> np.uint64(27)) * u(q)
+    xs = np.arange(1 << 16, dtype=np.uint64)
+    b16 = barrett16(xs)
+    assert (b16 % u(q) == xs % u(q)).all() and (b16 <= q + 1).all()
+    assert np.flatnonzero(b16 == q + 1).tolist() == [56594, 59923, 63252]
+    assert (b16[:16 * q] <= q).all()
+    # canon16 = csubq(barrett16) on every x < 2^17: exact exactly up to 106529 (where x 40317 still fits 32 bits), which
+    # covers its callers: 4096 + 14q = 50702 (ntt_warp), 16 (q - 1) = 53248 (k_vecmul_batch at k = 16), 2 * 4095 (poly_add)
+    x17 = np.arange(1 << 17, dtype=np.uint64)
+    b = barrett16(x17)
+    c16 = np.minimum(b, b - u(q))  # csubq: a wrapped r - q is large
+    exact = c16 == x17 % u(q)
+    assert exact[:106530].all() and not exact[106530]
+    assert max(4096 + 14 * q, 16 * (q - 1), 2 * 4095) <= 106529
+    # mul_shoup (16-bit Shoup word) on every a < 2^16 with every zeta and both inverse-last words: congruent, < 2q
+    a16 = np.arange(1 << 16, dtype=np.uint64)[:, None]
+    ws = np.concatenate([zetas, u([zetas[1] * u(3303) % u(q), 3303])])
+    r = (a16 * ws - ((a16 * ((ws << np.uint64(16)) // u(q))) >> np.uint64(16)) * u(q)) & u(0xFFFFFFFF)
+    assert (r < 2 * q).all() and (r % u(q) == a16 * ws % u(q)).all()
     # nibble j of a word by multiply (2^(28-4j)) and multiply-high (2^4)
     w = rng.integers(0, 1 << 32, 4096, dtype=np.uint64)
     for j in range(8):
