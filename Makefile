@@ -2,6 +2,7 @@
 #   make            -> crystals-kyber_b200/libmlkem_b200.so + build/microbench + oracle/
 #   make lib        -> only the product library
 #   make contracts  -> build/libmlkem_b200_contracts.so, the test-only harness of the device functions (tests/csrc/)
+#   make dropin     -> build/libref_dropin.so, oracle/ref_shim.c linked against the library (tests/csrc/dropin/)
 NVCC    ?= /usr/local/cuda/bin/nvcc
 ARCH    := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS := $(ARCH) -O3 -std=c++17 -lineinfo -Xcompiler -fPIC,-fvisibility=hidden -cudart static
@@ -9,7 +10,7 @@ PKG     := crystals-kyber_b200
 CSRC    := $(PKG)/csrc
 LIB     := $(PKG)/libmlkem_b200.so
 
-all: lib contracts tools examples oracle
+all: lib contracts dropin tools examples oracle
 
 lib: $(LIB)
 
@@ -21,6 +22,15 @@ contracts: build/libmlkem_b200_contracts.so
 build/libmlkem_b200_contracts.so: tests/csrc/device_contracts.cu $(CSRC)/mlkem_device.cuh $(CSRC)/mlkem_tables.inl
 	mkdir -p build
 	$(NVCC) $(NVFLAGS) -shared -o $@ tests/csrc/device_contracts.cu
+
+# test-only: the unmodified oracle/ref_shim.c, which recorded the golden vectors from the reference, built against the
+# drop-in API instead (tests/csrc/dropin/ml_kem.c stands in for the reference's ml_kem.c; tests/test_dropin_api_*.py)
+DROPIN_SO ?= build/libref_dropin.so
+dropin: $(DROPIN_SO)
+$(DROPIN_SO): oracle/ref_shim.c tests/csrc/dropin/ml_kem.c include/ml_kem.h include/sha3.h include/mlkem_b200.h $(LIB)
+	mkdir -p $(dir $@)
+	gcc -O2 -Wall -Werror -fPIC -shared -fvisibility=hidden -Itests/csrc/dropin -Iinclude -o $@ oracle/ref_shim.c \
+	    -L$(PKG) -lmlkem_b200 -Wl,-rpath,'$$ORIGIN/../$(PKG)' -lpthread
 
 # experiment build of the library (timing experiments that break the results on purpose: tools/time_encaps.py)
 exp: build/libmlkem_b200_exp.so
@@ -53,7 +63,7 @@ oracle: lib
 	$(MAKE) -C oracle drivers
 
 clean:
-	rm -f $(LIB) build/libmlkem_b200_contracts.so build/microbench build/keccak_bench build/coissue_bench
+	rm -f $(LIB) build/libmlkem_b200_contracts.so build/libref_dropin.so build/microbench build/keccak_bench build/coissue_bench
 	$(MAKE) -C oracle clean
 
-.PHONY: all lib contracts exp tools examples oracle clean
+.PHONY: all lib contracts dropin exp tools examples oracle clean
