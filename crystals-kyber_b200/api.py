@@ -394,6 +394,63 @@ class MLKEM:
         self._check(rc, "mlkem_b200_keys_generate")
         return KeyTable(self, handle, ps, o.device)
 
+    # ------------------------------------------------------------------ X25519 and the X25519MLKEM768 hybrid (ML-KEM in FIPS 203 mode)
+    # Sizes: client share 1216 = ek || X25519 public key, client secret 2432 = dk || X25519 scalar, server share 1120 = c || X25519
+    # public key, shared secret 64 = K || X25519 shared secret.  status per item: 0, -4 (ek fails the modulus check, encaps only) or
+    # -6 (all-zero X25519 shared secret); a failed item's outputs are zero.
+    def x25519(self, scalar, u=None):
+        """RFC 7748 X25519(scalar, u) for n x 32 byte rows; u=None: the base point 9 (public keys) -- mlkem_b200_x25519_batch."""
+        n = self._count(scalar, 32)
+        if u is None:
+            return self._call("mlkem_b200_x25519_batch", (n,), [(scalar, np.uint8), (None, np.uint8)], [((n, 32), np.uint8)])
+        return self._call("mlkem_b200_x25519_batch", (n,), [(scalar, np.uint8), (u, np.uint8)], [((n, 32), np.uint8)])
+
+    def x25519mlkem768_keygen(self, d, z, x_sk):
+        """Returns (client_share, client_secret) -- mlkem_b200_x25519mlkem768_keygen_batch."""
+        n = self._count(d, 32)
+        return self._call("mlkem_b200_x25519mlkem768_keygen_batch", (n,), [(d, np.uint8), (z, np.uint8), (x_sk, np.uint8)],
+                          [((n, 1216), np.uint8), ((n, 2432), np.uint8)])
+
+    def x25519mlkem768_encaps(self, client_share, m, x_eph):
+        """Returns (server_share, ss, status) -- mlkem_b200_x25519mlkem768_encaps_batch."""
+        n = self._count(m, 32)
+        return self._call("mlkem_b200_x25519mlkem768_encaps_batch", (n,), [(client_share, np.uint8), (m, np.uint8), (x_eph, np.uint8)],
+                          [((n, 1120), np.uint8), ((n, 64), np.uint8), ((n,), np.int32)])
+
+    def x25519mlkem768_decaps(self, client_secret, server_share):
+        """Returns (ss, status) -- mlkem_b200_x25519mlkem768_decaps_batch."""
+        n = self._count(server_share, 1120)
+        return self._call("mlkem_b200_x25519mlkem768_decaps_batch", (n,), [(client_secret, np.uint8), (server_share, np.uint8)],
+                          [((n, 64), np.uint8), ((n,), np.int32)])
+
+    def x25519mlkem768_keygen_seeded(self, n, seed=None, device=False):
+        """(client_share, client_secret) with (d_j, z_j, x_sk_j) expanded on the GPU -- mlkem_b200_x25519mlkem768_keygen_seeded_batch.
+        numpy, or with device=True torch CUDA tensors filled on the current torch stream."""
+        (cs, sec), o, ptr = self._out_opts(device, [(n, 1216), (n, 2432)])
+        rc = self.lib.mlkem_b200_x25519mlkem768_keygen_seeded_batch(n, _seed_ptr(seed), ptr(cs), ptr(sec), C.byref(o))
+        self._check(rc, "mlkem_b200_x25519mlkem768_keygen_seeded_batch")
+        return cs, sec
+
+    def x25519mlkem768_encaps_seeded(self, client_share, seed=None):
+        """(server_share, ss, status) with (m_j, x_eph_j) expanded on the GPU -- mlkem_b200_x25519mlkem768_encaps_seeded_batch.
+        A numpy client_share is host memory, a torch one device memory."""
+        if _is_torch(client_share):
+            import torch
+
+            client_share = client_share.contiguous()
+            n = client_share.numel() // 1216
+            (share, ss), o, ptr = self._out_opts(True, [(n, 1120), (n, 64)], client_share.device.index)
+            status = torch.empty(n, dtype=torch.int32, device=client_share.device)
+        else:
+            client_share = np.ascontiguousarray(client_share, np.uint8)
+            n = client_share.size // 1216
+            (share, ss), o, ptr = self._out_opts(False, [(n, 1120), (n, 64)])
+            status = np.empty(n, np.int32)
+        rc = self.lib.mlkem_b200_x25519mlkem768_encaps_seeded_batch(n, ptr(client_share), _seed_ptr(seed), ptr(share), ptr(ss), ptr(status),
+                                                                    C.byref(o))
+        self._check(rc, "mlkem_b200_x25519mlkem768_encaps_seeded_batch")
+        return share, ss, status
+
     # ------------------------------------------------------------------ K-PKE
     def pke_keygen(self, ps, d):
         sz, n = sizes(ps), self._count(d, 32)

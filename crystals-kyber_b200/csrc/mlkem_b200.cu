@@ -1802,6 +1802,157 @@ int mlkem_b200_tables(uint16_t zeta[128], uint16_t gamma[128]) {
 
 }  // extern "C"
 
+// ---- X25519 and the X25519MLKEM768 hybrid (draft-ietf-tls-ecdhe-mlkem) ----------------------------------------------------------
+// The ML-KEM kernels read ek / dk / c at their fixed strides, so each chunk gets dense images of them in its workspace: the rows
+// are copied out of (and into) the wire formats with k_scatter_rows (identity KeySel), k_x25519 reads and writes the X25519 parts
+// in place, and k_hybrid_join assembles the shared secret and the server share under the per-item status.
+namespace {
+
+constexpr uint32_t kSeedTagX25519KeyGen = 3, kSeedTagX25519Encaps = 4;
+
+int copy_rows(cudaStream_t st, int n, const uint8_t *src, size_t src_stride, uint8_t *dst, size_t dst_stride, size_t row_bytes) {
+    const size_t words = (size_t)n * (row_bytes / 16);
+    LAUNCH(k_scatter_rows, std::min<unsigned>(cdiv(words, 256), 148 * 16), 256, 0, st, n, (int)(row_bytes / 16), src, src_stride, KeySel{}, dst,
+           dst_stride);
+    return 0;
+}
+
+int launch_x25519(cudaStream_t st, int n, const uint8_t *scalar, size_t scalar_stride, const uint8_t *u, size_t u_stride, uint8_t *out,
+                  size_t out_stride, int *status) {
+    LAUNCH(k_x25519, std::min<unsigned>(cdiv(n, kX25519TPB), 148 * 32), kX25519TPB, 0, st, n, scalar, scalar_stride, u, u_stride, out,
+           out_stride, status);
+    return 0;
+}
+
+int launch_join(cudaStream_t st, int n, const int *st1, const int *st2, int *status, const uint8_t *K, const uint8_t *xss, uint8_t *ss,
+                const uint8_t *c, uint8_t *share) {
+    const size_t words = (size_t)n * (4 + (share ? MLKEM_B200_X25519MLKEM768_SERVER_SHARE_BYTES / 16 : 0));
+    LAUNCH(k_hybrid_join, std::min<unsigned>(cdiv(words, 256), 148 * 16), 256, 0, st, n, st1, st2, status, K, xss, ss, c, share);
+    return 0;
+}
+
+constexpr size_t kHybridWs = ws_bytes_per_item<P768>() + MLKEM_B200_X25519MLKEM768_CLIENT_SECRET_BYTES + 1184 + 1088 + 32 + 32 + 4 + 4;
+
+// KeyGen of the hybrid from (d, z, x_sk) in device memory: ek, dk into the workspace, then into the wire formats.
+int hybrid_keygen(cudaStream_t st, Arena &ws, int n, const uint8_t *d, const uint8_t *z, const uint8_t *x_sk, size_t x_sk_stride, uint8_t *share,
+                  uint8_t *secret, int gl) {
+    uint8_t *ek = ws.take<uint8_t>((size_t)n * P768::EK), *dk = ws.take<uint8_t>((size_t)n * P768::DK);
+    if (int rc = enqueue_keygen<P768>(st, ws, n, d, z, ek, dk, gl, true)) return rc;
+    if (int rc = copy_rows(st, n, ek, P768::EK, share, kHybridClientShare, P768::EK)) return rc;
+    if (int rc = copy_rows(st, n, dk, P768::DK, secret, kHybridClientSecret, P768::DK)) return rc;
+    if (int rc = copy_rows(st, n, x_sk, x_sk_stride, secret + P768::DK, kHybridClientSecret, 32)) return rc;
+    return launch_x25519(st, n, x_sk, x_sk_stride, nullptr, 0, share + P768::EK, kHybridClientShare, nullptr);
+}
+
+// Encaps of the hybrid: the FIPS 203 modulus check of the ek part, Encaps_internal, the two scalar multiplications with x_eph.
+int hybrid_encaps(cudaStream_t st, Arena &ws, int n, const uint8_t *client_share, const uint8_t *m, const uint8_t *x_eph, size_t x_eph_stride,
+                  uint8_t *server_share, uint8_t *ss, int *status, int gl) {
+    uint8_t *ek = ws.take<uint8_t>((size_t)n * P768::EK), *c = ws.take<uint8_t>((size_t)n * P768::C);
+    uint8_t *K = ws.take<uint8_t>((size_t)n * 32), *xss = ws.take<uint8_t>((size_t)n * 32);
+    int *st_mod = ws.take<int>(n), *st_x = ws.take<int>(n);
+    if (int rc = copy_rows(st, n, client_share, kHybridClientShare, ek, P768::EK, P768::EK)) return rc;
+    LAUNCH((k_check_ek_modulus<P768>), cdiv(n, kHashTPB), kHashTPB, 0, st, n, ek, st_mod);
+    if (int rc = enqueue_encaps<P768>(st, ws, n, ek, m, c, K, gl, true)) return rc;
+    if (int rc = launch_x25519(st, n, x_eph, x_eph_stride, nullptr, 0, server_share + P768::C, kHybridServerShare, nullptr)) return rc;
+    if (int rc = launch_x25519(st, n, x_eph, x_eph_stride, client_share + P768::EK, kHybridClientShare, xss, 32, st_x)) return rc;
+    return launch_join(st, n, st_mod, st_x, status, K, xss, ss, c, server_share);
+}
+
+}  // namespace
+
+extern "C" {
+
+int mlkem_b200_x25519_batch(size_t n, const uint8_t *scalar, const uint8_t *u, uint8_t *out, const mlkem_b200_opts *o) {
+    std::vector<Buf> bufs = {{scalar, nullptr, 32}, {nullptr, out, 32}};
+    const bool has_u = u != nullptr;
+    if (has_u) bufs.push_back({u, nullptr, 32});
+    return drive(o, n, 0, bufs, [=](cudaStream_t st, Arena &, int cn, void **p, size_t) {
+        return launch_x25519(st, cn, (const uint8_t *)p[0], 32, has_u ? (const uint8_t *)p[2] : nullptr, 32, (uint8_t *)p[1], 32, nullptr);
+    });
+}
+
+int mlkem_b200_x25519mlkem768_keygen_batch(size_t n, const uint8_t *d, const uint8_t *z, const uint8_t *x_sk, uint8_t *client_share,
+                                           uint8_t *client_secret, const mlkem_b200_opts *o) {
+    const int gl = group_limit_of(o);
+    return drive(o, n, kHybridWs,
+                 {{d, nullptr, 32}, {z, nullptr, 32}, {x_sk, nullptr, 32}, {nullptr, client_share, kHybridClientShare},
+                  {nullptr, client_secret, kHybridClientSecret}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     return hybrid_keygen(st, ws, cn, (const uint8_t *)p[0], (const uint8_t *)p[1], (const uint8_t *)p[2], 32, (uint8_t *)p[3],
+                                          (uint8_t *)p[4], gl);
+                 });
+}
+
+int mlkem_b200_x25519mlkem768_encaps_batch(size_t n, const uint8_t *client_share, const uint8_t *m, const uint8_t *x_eph, uint8_t *server_share,
+                                           uint8_t *ss, int32_t *status, const mlkem_b200_opts *o) {
+    const int gl = group_limit_of(o);
+    return drive(o, n, kHybridWs,
+                 {{client_share, nullptr, kHybridClientShare}, {m, nullptr, 32}, {x_eph, nullptr, 32}, {nullptr, server_share, kHybridServerShare},
+                  {nullptr, ss, kHybridSecret}, {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     return hybrid_encaps(st, ws, cn, (const uint8_t *)p[0], (const uint8_t *)p[1], (const uint8_t *)p[2], 32, (uint8_t *)p[3],
+                                          (uint8_t *)p[4], (int *)p[5], gl);
+                 });
+}
+
+int mlkem_b200_x25519mlkem768_decaps_batch(size_t n, const uint8_t *client_secret, const uint8_t *server_share, uint8_t *ss, int32_t *status,
+                                           const mlkem_b200_opts *o) {
+    const int gl = group_limit_of(o);
+    return drive(o, n, kHybridWs,
+                 {{client_secret, nullptr, kHybridClientSecret}, {server_share, nullptr, kHybridServerShare}, {nullptr, ss, kHybridSecret},
+                  {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     const uint8_t *secret = (const uint8_t *)p[0], *share = (const uint8_t *)p[1];
+                     uint8_t *dk = ws.take<uint8_t>((size_t)cn * P768::DK), *c = ws.take<uint8_t>((size_t)cn * P768::C);
+                     uint8_t *K = ws.take<uint8_t>((size_t)cn * 32), *xss = ws.take<uint8_t>((size_t)cn * 32);
+                     int *st_x = ws.take<int>(cn);
+                     if (int rc = copy_rows(st, cn, secret, kHybridClientSecret, dk, P768::DK, P768::DK)) return rc;
+                     if (int rc = copy_rows(st, cn, share, kHybridServerShare, c, P768::C, P768::C)) return rc;
+                     if (int rc = enqueue_decaps<P768>(st, ws, cn, dk, KeySel{}, c, K, gl, true)) return rc;
+                     if (int rc = launch_x25519(st, cn, secret + P768::DK, kHybridClientSecret, share + P768::C, kHybridServerShare, xss, 32, st_x))
+                         return rc;
+                     return launch_join(st, cn, st_x, nullptr, (int *)p[3], K, xss, (uint8_t *)p[2], nullptr, nullptr);
+                 });
+}
+
+int mlkem_b200_x25519mlkem768_keygen_seeded_batch(size_t n, const uint8_t *seed, uint8_t *client_share, uint8_t *client_secret,
+                                                  const mlkem_b200_opts *opts) {
+    const SyncOpts so(opts);
+    const mlkem_b200_opts *o = so.p;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        return drive(o, n, kHybridWs + 96, {{nullptr, client_share, kHybridClientShare}, {nullptr, client_secret, kHybridClientSecret}},
+                     [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                         uint8_t *d = ws.take<uint8_t>((size_t)cn * 32), *z = ws.take<uint8_t>((size_t)cn * 32), *x = ws.take<uint8_t>((size_t)cn * 32);
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagKeyGen, d, z)) return rc;
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagX25519KeyGen, x, nullptr)) return rc;
+                         return hybrid_keygen(st, ws, cn, d, z, x, 32, (uint8_t *)p[0], (uint8_t *)p[1], gl);
+                     });
+    });
+}
+
+int mlkem_b200_x25519mlkem768_encaps_seeded_batch(size_t n, const uint8_t *client_share, const uint8_t *seed, uint8_t *server_share, uint8_t *ss,
+                                                  int32_t *status, const mlkem_b200_opts *opts) {
+    const SyncOpts so(opts);
+    const mlkem_b200_opts *o = so.p;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        return drive(o, n, kHybridWs + 64,
+                     {{client_share, nullptr, kHybridClientShare}, {nullptr, server_share, kHybridServerShare}, {nullptr, ss, kHybridSecret},
+                      {nullptr, status, 4}},
+                     [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                         uint8_t *m = ws.take<uint8_t>((size_t)cn * 32), *x = ws.take<uint8_t>((size_t)cn * 32);
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagEncaps, m, nullptr)) return rc;
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagX25519Encaps, x, nullptr)) return rc;
+                         return hybrid_encaps(st, ws, cn, (const uint8_t *)p[0], m, x, 32, (uint8_t *)p[1], (uint8_t *)p[2], (int *)p[3], gl);
+                     });
+    });
+}
+
+}  // extern "C"
+
 #include "mlkem_profile.inl"
 #include "ml_kem_compat.inl"
 #include "sha3_compat.inl"

@@ -19,6 +19,7 @@
 // row and hash input is 8-byte aligned.
 #pragma once
 #include "mlkem_device.cuh"
+#include "x25519_device.cuh"
 
 namespace mlkem {
 
@@ -1721,6 +1722,66 @@ __global__ void __launch_bounds__(kPrimTPB) k_compress_batch(long long nvec, con
             w[k] = lo | (hi << 16);
         }
         out[i] = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+}
+
+// =================================================================================================
+// X25519 and the X25519MLKEM768 hybrid (draft-ietf-tls-ecdhe-mlkem)
+// =================================================================================================
+constexpr int kX25519TPB = 128;  // threads (= scalar multiplications) per block of k_x25519
+// Wire formats of X25519MLKEM768: the ML-KEM-768 part first, then the 32-byte X25519 part.  Every size and offset is a multiple
+// of 16, so rows stay 16-byte aligned.
+constexpr int kHybridClientShare = 1216, kHybridClientSecret = 2432, kHybridServerShare = 1120, kHybridSecret = 64;
+
+__device__ __forceinline__ void load_words32(const uint8_t *p, uint32_t w[8]) {
+    const uint4 a = __ldg(reinterpret_cast<const uint4 *>(p)), b = __ldg(reinterpret_cast<const uint4 *>(p) + 1);
+    w[0] = a.x, w[1] = a.y, w[2] = a.z, w[3] = a.w, w[4] = b.x, w[5] = b.y, w[6] = b.z, w[7] = b.w;
+}
+
+// out_i = X25519(scalar_i, u_i) (RFC 7748 section 5), one item per thread, grid-stride.  Rows are read and written at their own
+// strides (multiples of 16), so the kernel works straight on shares and secrets.  u == nullptr: the base point 9.  status (may be
+// null): status[i] = -6 when out_i is all zero (RFC 8446 section 7.4.2), else 0.
+__global__ void __launch_bounds__(kX25519TPB) k_x25519(int n, const uint8_t *__restrict__ scalar, size_t scalar_stride,
+                                                       const uint8_t *__restrict__ u, size_t u_stride, uint8_t *__restrict__ out,
+                                                       size_t out_stride, int *__restrict__ status) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        uint32_t k[8], uw[8] = {9, 0, 0, 0, 0, 0, 0, 0}, r[8];
+        load_words32(scalar + scalar_stride * i, k);
+        if (u) load_words32(u + u_stride * i, uw);
+        const uint32_t zero = x25519::scalarmult(r, k, uw);
+        uint4 *o = reinterpret_cast<uint4 *>(out + out_stride * i);
+        o[0] = make_uint4(r[0], r[1], r[2], r[3]);
+        o[1] = make_uint4(r[4], r[5], r[6], r[7]);
+        if (status) status[i] = -6 * (int)zero;
+    }
+}
+
+// The hybrid's outputs of item i from the dense images of its ML-KEM and X25519 halves, 16 bytes per thread, grid-stride:
+//   status_i = st1_i, or st2_i where st1_i == 0 (st2 may be null): the first failing check wins;
+//   ss_i = K_i || xss_i, and (share != null) share_i[0, 1088) = c_i -- share_i[1088, 1120) already holds the X25519 public key --
+//   all zero where status_i != 0.  The status selects by mask, not by branch.
+__global__ void __launch_bounds__(256) k_hybrid_join(int n, const int *__restrict__ st1, const int *__restrict__ st2, int *__restrict__ status,
+                                                     const uint8_t *__restrict__ K, const uint8_t *__restrict__ xss, uint8_t *__restrict__ ss,
+                                                     const uint8_t *__restrict__ c, uint8_t *__restrict__ share) {
+    constexpr int kCWords = 1088 / 16, kShareWords = kHybridServerShare / 16;
+    const int words = 4 + (share ? kShareWords : 0);
+    const size_t total = (size_t)n * words;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const int i = (int)(t / words), w = (int)(t - (size_t)i * words);
+        const int s1 = st1[i], s2 = st2 ? st2[i] : 0;
+        const int s = s1 | (s2 & -(int)(s1 == 0));
+        const uint32_t m = 0u - (uint32_t)(s == 0);
+        uint4 v;
+        if (w < 4) {
+            v = w < 2 ? reinterpret_cast<const uint4 *>(K + 32 * (size_t)i)[w] : reinterpret_cast<const uint4 *>(xss + 32 * (size_t)i)[w - 2];
+            if (w == 0) status[i] = s;
+        } else {
+            v = w - 4 < kCWords ? reinterpret_cast<const uint4 *>(c + 1088 * (size_t)i)[w - 4]
+                                : reinterpret_cast<const uint4 *>(share + (size_t)kHybridServerShare * i)[w - 4];
+        }
+        v = make_uint4(v.x & m, v.y & m, v.z & m, v.w & m);
+        if (w < 4) reinterpret_cast<uint4 *>(ss + (size_t)kHybridSecret * i)[w] = v;
+        else reinterpret_cast<uint4 *>(share + (size_t)kHybridServerShare * i)[w - 4] = v;
     }
 }
 

@@ -66,6 +66,12 @@ SIGNATURES = {
     "mlkem_b200_kem_encaps_keyed_batch": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _P8, _P8, _PO]),
     "mlkem_b200_keys_generate": (C.c_int, [C.c_int, C.c_size_t, _P8, _PO, C.POINTER(C.c_void_p)]),
     "mlkem_b200_keys_replace_generate": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, _P8, _PO]),
+    "mlkem_b200_x25519_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _PO]),
+    "mlkem_b200_x25519mlkem768_keygen_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, _P8, _PO]),
+    "mlkem_b200_x25519mlkem768_encaps_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_x25519mlkem768_decaps_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_x25519mlkem768_keygen_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _PO]),
+    "mlkem_b200_x25519mlkem768_encaps_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
     "mlkem_b200_pke_keygen_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _P8, _PO]),
     "mlkem_b200_pke_encrypt_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _P8, _P8, _PO]),
     "mlkem_b200_pke_decrypt_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, C.c_size_t, _P8, _P8, _PO]),

@@ -275,6 +275,60 @@ int mlkem_b200_keys_generate(int param_set, size_t n_keys, const uint8_t *seed, 
 int mlkem_b200_keys_replace_generate(mlkem_b200_keys *keys, size_t n, const uint32_t *slot, const uint8_t *seed,
                                      const mlkem_b200_opts *opts);
 
+/* ---- X25519 (RFC 7748) and the X25519MLKEM768 hybrid key exchange (draft-ietf-tls-ecdhe-mlkem, TLS group 0x11EC) ------------ */
+
+/* Wire formats of X25519MLKEM768, the ML-KEM-768 part first (every size and offset is a multiple of 16):
+ *   client share   ML-KEM-768 ek (1184)         || X25519 public key (32)
+ *   client secret  ML-KEM-768 dk (2400)         || X25519 private scalar (32, raw: clamped only inside X25519)
+ *   server share   ML-KEM-768 ciphertext (1088) || X25519 public key (32)
+ *   shared secret  ML-KEM shared secret (32)    || X25519 shared secret (32) */
+#define MLKEM_B200_X25519MLKEM768_CLIENT_SHARE_BYTES 1216
+#define MLKEM_B200_X25519MLKEM768_CLIENT_SECRET_BYTES 2432
+#define MLKEM_B200_X25519MLKEM768_SERVER_SHARE_BYTES 1120
+#define MLKEM_B200_X25519MLKEM768_SHARED_SECRET_BYTES 64
+#define MLKEM_B200_ERR_X25519_ZERO (-6) /* per-item status: the X25519 shared secret is all zero (RFC 8446 section 7.4.2) */
+
+/* X25519(k, u) of RFC 7748 section 5: the scalar is clamped, bit 255 of u is ignored and u in [p, 2^255) is accepted.
+ * scalar, u, out: n x 32.  u == NULL: the base point 9 (the public key of `scalar`).  No zero check: this is the primitive,
+ * an all-zero output (u of small order) is returned as it is.  Constant-flow on the device: no branch, trip count or memory
+ * index depends on the scalar or on u. */
+int mlkem_b200_x25519_batch(size_t n, const uint8_t *scalar, const uint8_t *u, uint8_t *out, const mlkem_b200_opts *opts);
+
+/* The three operations of X25519MLKEM768.  ML-KEM always runs in FIPS 203 mode here, whatever opts->flags says (the
+ * reference's SHAKE128 PRF / J would not interoperate); sample_group_limit, memory spaces, chunk_items, streams and
+ * MLKEM_B200_FLAG_ASYNC (host memory) behave as for the other calls.
+ *
+ * Per-item status instead of a whole-call error, so that one bad client cannot fail a batch of handshakes.  status is n x int32
+ * in opts->mem like the other buffers (device-memory calls stay asynchronous) and may not be NULL (MLKEM_B200_ERR_ARG):
+ *   encaps  MLKEM_B200_ERR_MODULUS (-4) when the ek part fails the FIPS 203 section 7.2 modulus check, else
+ *           MLKEM_B200_ERR_X25519_ZERO (-6) when the X25519 shared secret is all zero; the first failing check wins;
+ *   decaps  -6 only: ML-KEM decapsulation never fails (a tampered ciphertext gives the implicit-rejection key).
+ * A failed item's shared secret is all zero and, for encaps, so is its server share.  Every item is computed the same way
+ * whatever its status; only the outputs are masked.
+ *
+ * Secrets: dk and the X25519 scalars exist only in the caller's buffers and in the chunk workspaces (wiped when freed). */
+/* d, z, x_sk: n x 32.  client_share: n x 1216 = ek || X25519(x_sk, 9).  client_secret: n x 2432 = dk || x_sk.
+ * (ek, dk) = ML-KEM.KeyGen_internal(d, z) in FIPS 203 mode. */
+int mlkem_b200_x25519mlkem768_keygen_batch(size_t n, const uint8_t *d, const uint8_t *z, const uint8_t *x_sk,
+                                           uint8_t *client_share, uint8_t *client_secret, const mlkem_b200_opts *opts);
+/* client_share: n x 1216, m, x_eph: n x 32.  server_share: n x 1120 = c || X25519(x_eph, 9); ss: n x 64 = K ||
+ * X25519(x_eph, client X25519 key), (K, c) = ML-KEM.Encaps_internal(ek, m). */
+int mlkem_b200_x25519mlkem768_encaps_batch(size_t n, const uint8_t *client_share, const uint8_t *m, const uint8_t *x_eph,
+                                           uint8_t *server_share, uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts);
+/* client_secret: n x 2432, server_share: n x 1120.  ss: n x 64 = ML-KEM.Decaps_internal(dk, c) || X25519(x_sk, server key). */
+int mlkem_b200_x25519mlkem768_decaps_batch(size_t n, const uint8_t *client_secret, const uint8_t *server_share,
+                                           uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts);
+/* Randomness expanded on the device, as mlkem_b200_kem_*_seeded_batch (seed: HOST memory, 32 bytes or NULL = 32 bytes of
+ * /dev/urandom per call; synchronous in both memory spaces, MLKEM_B200_FLAG_ASYNC ignored; the seed is wiped):
+ *   keygen  (d_j, z_j) = R_j of tag 1 (exactly as mlkem_b200_kem_keygen_seeded_batch), x_sk_j = R_j[0..32) of tag 3;
+ *   encaps  m_j = R_j[0..32) of tag 2 (exactly as mlkem_b200_kem_encaps_seeded_batch), x_eph_j = R_j[0..32) of tag 4.
+ * No expanded secret crosses PCIe towards the device. */
+int mlkem_b200_x25519mlkem768_keygen_seeded_batch(size_t n, const uint8_t *seed, uint8_t *client_share,
+                                                  uint8_t *client_secret, const mlkem_b200_opts *opts);
+int mlkem_b200_x25519mlkem768_encaps_seeded_batch(size_t n, const uint8_t *client_share, const uint8_t *seed,
+                                                  uint8_t *server_share, uint8_t *ss, int32_t *status,
+                                                  const mlkem_b200_opts *opts);
+
 /* ---- K-PKE (FIPS 203 Alg. 13-15) -------------------------------------------------------------------- */
 
 /* PKE_KeyGen, ml_kem.c:651.  d: n x 32.  ek: n x (384k+32).  dk_pke: n x 384k. */
