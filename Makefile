@@ -1,8 +1,8 @@
 # Top-level build: the product library (CUDA, sm_100a), the INT32 microbenchmark and the checkers.
 #   make            -> crystals-kyber_b200/libmlkem_b200.so + build/microbench + oracle/
 #   make lib        -> only the product library
-#   make contracts  -> build/libmlkem_b200_contracts.so and build/libx25519_contracts.so, the test-only harnesses of the device
-#                      functions (tests/csrc/)
+#   make contracts  -> build/libmlkem_b200_contracts.so, build/libx25519_contracts.so and build/libp256_contracts.so, the
+#                      test-only harnesses of the device functions (tests/csrc/)
 #   make dropin     -> build/libref_dropin.so, oracle/ref_shim.c linked against the library (tests/csrc/dropin/)
 NVCC    ?= /usr/local/cuda/bin/nvcc
 ARCH    := -gencode arch=compute_100a,code=sm_100a
@@ -15,11 +15,11 @@ all: lib contracts dropin tools examples oracle
 
 lib: $(LIB)
 
-$(LIB): $(CSRC)/mlkem_b200.cu $(CSRC)/mlkem_kernels.cuh $(CSRC)/mlkem_device.cuh $(CSRC)/x25519_device.cuh $(CSRC)/ml_kem_compat.inl $(CSRC)/mlkem_profile.inl $(CSRC)/sha3_compat.inl $(CSRC)/mlkem_tables.inl include/mlkem_b200.h include/ml_kem.h include/sha3.h
+$(LIB): $(CSRC)/mlkem_b200.cu $(CSRC)/mlkem_kernels.cuh $(CSRC)/mlkem_device.cuh $(CSRC)/x25519_device.cuh $(CSRC)/p256_device.cuh $(CSRC)/ml_kem_compat.inl $(CSRC)/mlkem_profile.inl $(CSRC)/sha3_compat.inl $(CSRC)/mlkem_tables.inl include/mlkem_b200.h include/ml_kem.h include/sha3.h
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(CSRC)/mlkem_b200.cu
 
 # test-only harness: the device functions of mlkem_device.cuh one by one, on the library's tables (tests/test_device_contracts_gpu.py)
-contracts: build/libmlkem_b200_contracts.so build/libx25519_contracts.so
+contracts: build/libmlkem_b200_contracts.so build/libx25519_contracts.so build/libp256_contracts.so
 build/libmlkem_b200_contracts.so: tests/csrc/device_contracts.cu $(CSRC)/mlkem_device.cuh $(CSRC)/mlkem_tables.inl
 	mkdir -p build
 	$(NVCC) $(NVFLAGS) -shared -o $@ tests/csrc/device_contracts.cu
@@ -27,6 +27,10 @@ build/libmlkem_b200_contracts.so: tests/csrc/device_contracts.cu $(CSRC)/mlkem_d
 build/libx25519_contracts.so: tests/csrc/x25519_contracts.cu $(CSRC)/x25519_device.cuh
 	mkdir -p build
 	$(NVCC) $(NVFLAGS) -shared -o $@ tests/csrc/x25519_contracts.cu
+# the same for the field, point and scalar functions of p256_device.cuh (tests/test_p256_contracts_gpu.py)
+build/libp256_contracts.so: tests/csrc/p256_contracts.cu $(CSRC)/p256_device.cuh
+	mkdir -p build
+	$(NVCC) $(NVFLAGS) -shared -o $@ tests/csrc/p256_contracts.cu
 
 # test-only: the unmodified oracle/ref_shim.c, which recorded the golden vectors from the reference, built against the
 # drop-in API instead (tests/csrc/dropin/ml_kem.c stands in for the reference's ml_kem.c; tests/test_dropin_api_*.py)
@@ -68,7 +72,7 @@ oracle: lib
 	$(MAKE) -C oracle drivers
 
 clean:
-	rm -f $(LIB) build/libmlkem_b200_contracts.so build/libx25519_contracts.so build/libref_dropin.so build/microbench build/keccak_bench build/coissue_bench
+	rm -f $(LIB) build/libmlkem_b200_contracts.so build/libx25519_contracts.so build/libp256_contracts.so build/libref_dropin.so build/microbench build/keccak_bench build/coissue_bench
 	$(MAKE) -C oracle clean
 
 .PHONY: all lib contracts dropin exp tools examples oracle clean

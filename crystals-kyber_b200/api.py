@@ -451,6 +451,67 @@ class MLKEM:
         self._check(rc, "mlkem_b200_x25519mlkem768_encaps_seeded_batch")
         return share, ss, status
 
+    # ------------------------------------------------------------------ P-256 and the SecP256r1MLKEM768 hybrid (ML-KEM in FIPS 203 mode)
+    # The P-256 part comes first: client share 1249 = P-256 point || ek, server share 1153 = P-256 point || c, shared secret 64 =
+    # ECDH secret || K; client secret 2432 = dk || P-256 scalar.  Points are 65 bytes (0x04 || X || Y), scalars 32 bytes, both
+    # big-endian.  status per item: 0, -7 (own scalar outside [1, n - 1]), -4 (ek fails the modulus check, encaps only) or -8
+    # (peer point invalid), the first failing check in that order; a failed item's outputs are zero.
+    def p256_public(self, scalar):
+        """(pub, status): scalar G as 65-byte points for n x 32 byte scalars -- mlkem_b200_p256_public_batch."""
+        n = self._count(scalar, 32)
+        return self._call("mlkem_b200_p256_public_batch", (n,), [(scalar, np.uint8)], [((n, 65), np.uint8), ((n,), np.int32)])
+
+    def p256_ecdh(self, scalar, peer):
+        """(ss, status): the 32-byte X of scalar peer, peer as n x 65 byte points -- mlkem_b200_p256_ecdh_batch."""
+        n = self._count(scalar, 32)
+        return self._call("mlkem_b200_p256_ecdh_batch", (n,), [(scalar, np.uint8), (peer, np.uint8)], [((n, 32), np.uint8), ((n,), np.int32)])
+
+    def secp256r1mlkem768_keygen(self, d, z, ec_sk):
+        """Returns (client_share, client_secret, status) -- mlkem_b200_secp256r1mlkem768_keygen_batch."""
+        n = self._count(d, 32)
+        return self._call("mlkem_b200_secp256r1mlkem768_keygen_batch", (n,), [(d, np.uint8), (z, np.uint8), (ec_sk, np.uint8)],
+                          [((n, 1249), np.uint8), ((n, 2432), np.uint8), ((n,), np.int32)])
+
+    def secp256r1mlkem768_encaps(self, client_share, m, ec_eph):
+        """Returns (server_share, ss, status) -- mlkem_b200_secp256r1mlkem768_encaps_batch."""
+        n = self._count(m, 32)
+        return self._call("mlkem_b200_secp256r1mlkem768_encaps_batch", (n,), [(client_share, np.uint8), (m, np.uint8), (ec_eph, np.uint8)],
+                          [((n, 1153), np.uint8), ((n, 64), np.uint8), ((n,), np.int32)])
+
+    def secp256r1mlkem768_decaps(self, client_secret, server_share):
+        """Returns (ss, status) -- mlkem_b200_secp256r1mlkem768_decaps_batch."""
+        n = self._count(server_share, 1153)
+        return self._call("mlkem_b200_secp256r1mlkem768_decaps_batch", (n,), [(client_secret, np.uint8), (server_share, np.uint8)],
+                          [((n, 64), np.uint8), ((n,), np.int32)])
+
+    def secp256r1mlkem768_keygen_seeded(self, n, seed=None, device=False):
+        """(client_share, client_secret) with (d_j, z_j, ec_sk_j) expanded on the GPU -- mlkem_b200_secp256r1mlkem768_keygen_seeded_batch.
+        numpy, or with device=True torch CUDA tensors filled on the current torch stream."""
+        (cs, sec), o, ptr = self._out_opts(device, [(n, 1249), (n, 2432)])
+        rc = self.lib.mlkem_b200_secp256r1mlkem768_keygen_seeded_batch(n, _seed_ptr(seed), ptr(cs), ptr(sec), C.byref(o))
+        self._check(rc, "mlkem_b200_secp256r1mlkem768_keygen_seeded_batch")
+        return cs, sec
+
+    def secp256r1mlkem768_encaps_seeded(self, client_share, seed=None):
+        """(server_share, ss, status) with (m_j, ec_eph_j) expanded on the GPU -- mlkem_b200_secp256r1mlkem768_encaps_seeded_batch.
+        A numpy client_share is host memory, a torch one device memory."""
+        if _is_torch(client_share):
+            import torch
+
+            client_share = client_share.contiguous()
+            n = client_share.numel() // 1249
+            (share, ss), o, ptr = self._out_opts(True, [(n, 1153), (n, 64)], client_share.device.index)
+            status = torch.empty(n, dtype=torch.int32, device=client_share.device)
+        else:
+            client_share = np.ascontiguousarray(client_share, np.uint8)
+            n = client_share.size // 1249
+            (share, ss), o, ptr = self._out_opts(False, [(n, 1153), (n, 64)])
+            status = np.empty(n, np.int32)
+        rc = self.lib.mlkem_b200_secp256r1mlkem768_encaps_seeded_batch(n, ptr(client_share), _seed_ptr(seed), ptr(share), ptr(ss), ptr(status),
+                                                                       C.byref(o))
+        self._check(rc, "mlkem_b200_secp256r1mlkem768_encaps_seeded_batch")
+        return share, ss, status
+
     # ------------------------------------------------------------------ K-PKE
     def pke_keygen(self, ps, d):
         sz, n = sizes(ps), self._count(d, 32)

@@ -1953,6 +1953,189 @@ int mlkem_b200_x25519mlkem768_encaps_seeded_batch(size_t n, const uint8_t *clien
 
 }  // extern "C"
 
+// ---- P-256 and the SecP256r1MLKEM768 hybrid (draft-ietf-tls-ecdhe-mlkem) ----------------------------------------------------
+// The same structure as the X25519 hybrid, with the ECDH part first in every wire format.  The share rows (1249, 1153 bytes) and
+// the 65-byte points are not multiples of 16, so ek and c move between them and the dense images with k_copy_bytes; dk still
+// moves with k_scatter_rows (offset 0 of a 2432-byte row).  k_p256 reads and writes the P-256 parts in place and k_p256_join
+// assembles the shared secret and the server share under the per-item status.
+namespace {
+
+constexpr uint32_t kSeedTagP256KeyGen = 5, kSeedTagP256Encaps = 6;
+
+// The options of a call with 65 / 1249 / 1153-byte rows: a caller's chunk_items is rounded up to a multiple of 16, so that every
+// chunk of a device-memory call starts 16-byte aligned (16 rows of any size do); the default chunk sizes and drive()'s halving
+// rule already are multiples of 16.  sync: MLKEM_B200_FLAG_ASYNC is dropped as in SyncOpts.
+struct OddRowOpts {
+    mlkem_b200_opts v;
+    const mlkem_b200_opts *p;
+    OddRowOpts(const mlkem_b200_opts *o, bool sync) : v(o ? *o : mlkem_b200_opts{-1, MLKEM_B200_MEM_HOST, nullptr, 0, 0, 0}), p(o ? &v : nullptr) {
+        if (v.chunk_items > 0) v.chunk_items = (int)std::min<long long>(((long long)v.chunk_items + 15) & ~15ll, 1 << 30);
+        if (sync) v.flags &= ~MLKEM_B200_FLAG_ASYNC;
+    }
+};
+
+int copy_bytes(cudaStream_t st, int n, const uint8_t *src, size_t src_stride, uint8_t *dst, size_t dst_stride, int row_bytes,
+               const int *status) {
+    LAUNCH(k_copy_bytes, std::min<unsigned>(cdiv(n, 8), 148 * 16), 256, 0, st, n, row_bytes, src, src_stride, dst, dst_stride, status);
+    return 0;
+}
+
+int launch_p256(cudaStream_t st, int n, const uint8_t *scalar, size_t scalar_stride, const uint8_t *point, size_t point_stride, uint8_t *out,
+                size_t out_stride, bool x_only, int *status) {
+    LAUNCH(k_p256, std::min<unsigned>(cdiv(n, kP256TPB), 148 * 32), kP256TPB, 0, st, n, scalar, scalar_stride, point, point_stride, out, out_stride,
+           (int)x_only, status);
+    return 0;
+}
+
+int launch_p256_join(cudaStream_t st, int n, const int *st_ec, const int *st_mod, int *status, const uint8_t *ecdh, const uint8_t *K, uint8_t *ss,
+                     const uint8_t *c, uint8_t *share) {
+    LAUNCH(k_p256_join, std::min<unsigned>(cdiv(n, 8), 148 * 16), 256, 0, st, n, st_ec, st_mod, status, ecdh, K, ss, c, share);
+    return 0;
+}
+
+// The scalars of a seeded call: R_j[0, 40) of `tag`, reduced by FIPS 186-5 A.2.1.
+int expand_p256_scalar(cudaStream_t st, Arena &ws, int n, const uint8_t *seed, size_t first, uint32_t tag, uint8_t *d) {
+    uint8_t *hi = ws.take<uint8_t>((size_t)n * 32), *lo = ws.take<uint8_t>((size_t)n * 32);
+    if (int rc = expand_seed(st, n, seed, first, tag, hi, lo)) return rc;
+    LAUNCH(k_p256_seed_scalar, cdiv(n, kHashTPB), kHashTPB, 0, st, n, hi, lo, d);
+    return 0;
+}
+
+// dense ek, dk and c, K, the ECDH secret and two status words per item, plus the seeded calls' scalars and seed expansions
+constexpr size_t kSecpWs = ws_bytes_per_item<P768>() + P768::DK + P768::EK + P768::C + 32 + 32 + 4 + 4 + 5 * 32;
+
+// KeyGen of the hybrid from (d, z, sk) in device memory: ek, dk into the workspace, then into the wire formats under the status
+// of the scalar check (-7).
+int secp_keygen(cudaStream_t st, Arena &ws, int n, const uint8_t *d, const uint8_t *z, const uint8_t *sk, size_t sk_stride, uint8_t *share,
+                uint8_t *secret, int *status, int gl) {
+    uint8_t *ek = ws.take<uint8_t>((size_t)n * P768::EK), *dk = ws.take<uint8_t>((size_t)n * P768::DK);
+    if (int rc = enqueue_keygen<P768>(st, ws, n, d, z, ek, dk, gl, true)) return rc;
+    if (int rc = launch_p256(st, n, sk, sk_stride, nullptr, 0, share, kSecpClientShare, false, status)) return rc;
+    if (int rc = copy_bytes(st, n, ek, P768::EK, share + kP256Point, kSecpClientShare, P768::EK, status)) return rc;
+    if (int rc = copy_bytes(st, n, dk, P768::DK, secret, kSecpClientSecret, P768::DK, status)) return rc;
+    return copy_bytes(st, n, sk, sk_stride, secret + P768::DK, kSecpClientSecret, 32, status);
+}
+
+// Encaps of the hybrid: the FIPS 203 modulus check of the ek part, Encaps_internal, the two scalar multiplications with eph.
+int secp_encaps(cudaStream_t st, Arena &ws, int n, const uint8_t *client_share, const uint8_t *m, const uint8_t *eph, size_t eph_stride,
+                uint8_t *server_share, uint8_t *ss, int *status, int gl) {
+    uint8_t *ek = ws.take<uint8_t>((size_t)n * P768::EK), *c = ws.take<uint8_t>((size_t)n * P768::C);
+    uint8_t *K = ws.take<uint8_t>((size_t)n * 32), *ecdh = ws.take<uint8_t>((size_t)n * 32);
+    int *st_mod = ws.take<int>(n), *st_ec = ws.take<int>(n);
+    if (int rc = copy_bytes(st, n, client_share + kP256Point, kSecpClientShare, ek, P768::EK, P768::EK, nullptr)) return rc;
+    LAUNCH((k_check_ek_modulus<P768>), cdiv(n, kHashTPB), kHashTPB, 0, st, n, ek, st_mod);
+    if (int rc = enqueue_encaps<P768>(st, ws, n, ek, m, c, K, gl, true)) return rc;
+    if (int rc = launch_p256(st, n, eph, eph_stride, nullptr, 0, server_share, kSecpServerShare, false, nullptr)) return rc;
+    if (int rc = launch_p256(st, n, eph, eph_stride, client_share, kSecpClientShare, ecdh, 32, true, st_ec)) return rc;
+    return launch_p256_join(st, n, st_ec, st_mod, status, ecdh, K, ss, c, server_share);
+}
+
+}  // namespace
+
+extern "C" {
+
+int mlkem_b200_p256_public_batch(size_t n, const uint8_t *scalar, uint8_t *pub, int32_t *status, const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, false);
+    return drive(oo.p, n, 0, {{scalar, nullptr, 32}, {nullptr, pub, kP256Point}, {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &, int cn, void **p, size_t) {
+                     return launch_p256(st, cn, (const uint8_t *)p[0], 32, nullptr, 0, (uint8_t *)p[1], kP256Point, false, (int *)p[2]);
+                 });
+}
+
+int mlkem_b200_p256_ecdh_batch(size_t n, const uint8_t *scalar, const uint8_t *peer, uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, false);
+    return drive(oo.p, n, 0, {{scalar, nullptr, 32}, {peer, nullptr, kP256Point}, {nullptr, ss, 32}, {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &, int cn, void **p, size_t) {
+                     return launch_p256(st, cn, (const uint8_t *)p[0], 32, (const uint8_t *)p[1], kP256Point, (uint8_t *)p[2], 32, true, (int *)p[3]);
+                 });
+}
+
+int mlkem_b200_secp256r1mlkem768_keygen_batch(size_t n, const uint8_t *d, const uint8_t *z, const uint8_t *ec_sk, uint8_t *client_share,
+                                              uint8_t *client_secret, int32_t *status, const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, false);
+    const int gl = group_limit_of(oo.p);
+    return drive(oo.p, n, kSecpWs,
+                 {{d, nullptr, 32}, {z, nullptr, 32}, {ec_sk, nullptr, 32}, {nullptr, client_share, kSecpClientShare},
+                  {nullptr, client_secret, kSecpClientSecret}, {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     return secp_keygen(st, ws, cn, (const uint8_t *)p[0], (const uint8_t *)p[1], (const uint8_t *)p[2], 32, (uint8_t *)p[3],
+                                        (uint8_t *)p[4], (int *)p[5], gl);
+                 });
+}
+
+int mlkem_b200_secp256r1mlkem768_encaps_batch(size_t n, const uint8_t *client_share, const uint8_t *m, const uint8_t *ec_eph, uint8_t *server_share,
+                                              uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, false);
+    const int gl = group_limit_of(oo.p);
+    return drive(oo.p, n, kSecpWs,
+                 {{client_share, nullptr, kSecpClientShare}, {m, nullptr, 32}, {ec_eph, nullptr, 32}, {nullptr, server_share, kSecpServerShare},
+                  {nullptr, ss, kSecpSecret}, {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     return secp_encaps(st, ws, cn, (const uint8_t *)p[0], (const uint8_t *)p[1], (const uint8_t *)p[2], 32, (uint8_t *)p[3],
+                                        (uint8_t *)p[4], (int *)p[5], gl);
+                 });
+}
+
+int mlkem_b200_secp256r1mlkem768_decaps_batch(size_t n, const uint8_t *client_secret, const uint8_t *server_share, uint8_t *ss, int32_t *status,
+                                              const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, false);
+    const int gl = group_limit_of(oo.p);
+    return drive(oo.p, n, kSecpWs,
+                 {{client_secret, nullptr, kSecpClientSecret}, {server_share, nullptr, kSecpServerShare}, {nullptr, ss, kSecpSecret},
+                  {nullptr, status, 4}},
+                 [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t) {
+                     const uint8_t *secret = (const uint8_t *)p[0], *share = (const uint8_t *)p[1];
+                     uint8_t *dk = ws.take<uint8_t>((size_t)cn * P768::DK), *c = ws.take<uint8_t>((size_t)cn * P768::C);
+                     uint8_t *K = ws.take<uint8_t>((size_t)cn * 32), *ecdh = ws.take<uint8_t>((size_t)cn * 32);
+                     int *st_ec = ws.take<int>(cn);
+                     if (int rc = copy_rows(st, cn, secret, kSecpClientSecret, dk, P768::DK, P768::DK)) return rc;
+                     if (int rc = copy_bytes(st, cn, share + kP256Point, kSecpServerShare, c, P768::C, P768::C, nullptr)) return rc;
+                     if (int rc = enqueue_decaps<P768>(st, ws, cn, dk, KeySel{}, c, K, gl, true)) return rc;
+                     if (int rc = launch_p256(st, cn, secret + P768::DK, kSecpClientSecret, share, kSecpServerShare, ecdh, 32, true, st_ec))
+                         return rc;
+                     return launch_p256_join(st, cn, st_ec, nullptr, (int *)p[3], ecdh, K, (uint8_t *)p[2], nullptr, nullptr);
+                 });
+}
+
+int mlkem_b200_secp256r1mlkem768_keygen_seeded_batch(size_t n, const uint8_t *seed, uint8_t *client_share, uint8_t *client_secret,
+                                                     const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, true);
+    const mlkem_b200_opts *o = oo.p;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        return drive(o, n, kSecpWs, {{nullptr, client_share, kSecpClientShare}, {nullptr, client_secret, kSecpClientSecret}},
+                     [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                         uint8_t *d = ws.take<uint8_t>((size_t)cn * 32), *z = ws.take<uint8_t>((size_t)cn * 32), *sk = ws.take<uint8_t>((size_t)cn * 32);
+                         int *status = ws.take<int>(cn);  // always 0: A.2.1 scalars are in [1, n - 1]
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagKeyGen, d, z)) return rc;
+                         if (int rc = expand_p256_scalar(st, ws, cn, dseed, first, kSeedTagP256KeyGen, sk)) return rc;
+                         return secp_keygen(st, ws, cn, d, z, sk, 32, (uint8_t *)p[0], (uint8_t *)p[1], status, gl);
+                     });
+    });
+}
+
+int mlkem_b200_secp256r1mlkem768_encaps_seeded_batch(size_t n, const uint8_t *client_share, const uint8_t *seed, uint8_t *server_share,
+                                                     uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts) {
+    const OddRowOpts oo(opts, true);
+    const mlkem_b200_opts *o = oo.p;
+    if (n == 0) return MLKEM_B200_OK;
+    const int gl = group_limit_of(o);
+    return with_call_seed(o, seed, [&](const uint8_t *dseed) -> int {
+        return drive(o, n, kSecpWs,
+                     {{client_share, nullptr, kSecpClientShare}, {nullptr, server_share, kSecpServerShare}, {nullptr, ss, kSecpSecret},
+                      {nullptr, status, 4}},
+                     [=](cudaStream_t st, Arena &ws, int cn, void **p, size_t first) {
+                         uint8_t *m = ws.take<uint8_t>((size_t)cn * 32), *eph = ws.take<uint8_t>((size_t)cn * 32);
+                         if (int rc = expand_seed(st, cn, dseed, first, kSeedTagEncaps, m, nullptr)) return rc;
+                         if (int rc = expand_p256_scalar(st, ws, cn, dseed, first, kSeedTagP256Encaps, eph)) return rc;
+                         return secp_encaps(st, ws, cn, (const uint8_t *)p[0], m, eph, 32, (uint8_t *)p[1], (uint8_t *)p[2], (int *)p[3], gl);
+                     });
+    });
+}
+
+}  // extern "C"
+
 #include "mlkem_profile.inl"
 #include "ml_kem_compat.inl"
 #include "sha3_compat.inl"

@@ -20,6 +20,7 @@
 #pragma once
 #include "mlkem_device.cuh"
 #include "x25519_device.cuh"
+#include "p256_device.cuh"
 
 namespace mlkem {
 
@@ -1782,6 +1783,90 @@ __global__ void __launch_bounds__(256) k_hybrid_join(int n, const int *__restric
         v = make_uint4(v.x & m, v.y & m, v.z & m, v.w & m);
         if (w < 4) reinterpret_cast<uint4 *>(ss + (size_t)kHybridSecret * i)[w] = v;
         else reinterpret_cast<uint4 *>(share + (size_t)kHybridServerShare * i)[w - 4] = v;
+    }
+}
+
+// =================================================================================================
+// P-256 and the SecP256r1MLKEM768 hybrid (draft-ietf-tls-ecdhe-mlkem)
+// =================================================================================================
+constexpr int kP256TPB = 128;  // threads (= scalar multiplications) per block of k_p256
+// Wire formats of SecP256r1MLKEM768: the 65-byte P-256 point first, then the ML-KEM-768 part; the client secret (never on the
+// wire) is dk || scalar.  Shares are not multiples of 16 bytes, so their rows are moved with byte accesses (k_copy_bytes).
+constexpr int kP256Point = 65, kSecpClientShare = 1249, kSecpClientSecret = 2432, kSecpServerShare = 1153, kSecpSecret = 64;
+
+// out_i = scalar_i * Q_i on P-256, one item per thread, grid-stride.  scalar_i: 32 big-endian bytes.  point == nullptr: Q_i = G;
+// else Q_i is the 65-byte encoding at point + point_stride * i, validated by point_decode.  out_i: the 32-byte X (x_only) or the
+// 65-byte encoding of the result.  status_i = -7 when scalar_i is outside [1, n - 1], else -8 when Q_i is invalid, else 0;
+// out_i is all zero where status_i != 0, and status is written where it is not null.  Rows are read and written with byte
+// accesses at any offset and stride, so the kernel works straight on shares and secrets.  Every item runs the same
+// instructions whatever its scalar, point and status.
+__global__ void __launch_bounds__(kP256TPB) k_p256(int n, const uint8_t *__restrict__ scalar, size_t scalar_stride,
+                                                   const uint8_t *__restrict__ point, size_t point_stride, uint8_t *__restrict__ out,
+                                                   size_t out_stride, int x_only, int *__restrict__ status) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        uint32_t k[8], x[8], y[8];
+        p256::words_from_be(scalar + scalar_stride * i, k);
+        const uint32_t k_ok = p256::scalar_ok_mask(k);
+        p256::pt Q = p256::base_point();
+        const uint32_t q_ok = point ? p256::point_decode(point + point_stride * i, Q) : 0xFFFFFFFFu;
+        p256::to_affine(p256::scalarmult(k, Q), x, y);
+        const uint32_t m = k_ok & q_ok;
+        uint8_t *o = out + out_stride * i;
+        if (x_only) p256::words_to_be(x, o, m);
+        else p256::point_encode(x, y, o, m);
+        if (status) status[i] = (int)((~k_ok & (uint32_t)-7) | (k_ok & ~q_ok & (uint32_t)-8));
+    }
+}
+
+// d_i = (c_i mod (n - 1)) + 1 of FIPS 186-5 A.2.1 (p256::seed_scalar) as 32 big-endian bytes, where c_i = hi_i[0, 32) || lo_i[0, 8)
+// = R_j[0, 40) of k_expand_seed (out0 = hi, out1 = lo).  One item per thread; every row is 32 bytes.
+__global__ void __launch_bounds__(kHashTPB) k_p256_seed_scalar(int n, const uint8_t *__restrict__ hi, const uint8_t *__restrict__ lo,
+                                                               uint8_t *__restrict__ d) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t w[8];
+    p256::seed_scalar(hi + 32 * (size_t)i, lo + 32 * (size_t)i, w);
+    p256::words_to_be(w, d + 32 * (size_t)i, 0xFFFFFFFFu);
+}
+
+// dst_i[0, row_bytes) = src_i[0, row_bytes) for rows at any offset and stride -- the rows k_scatter_rows cannot move, whose
+// sizes or offsets are not multiples of 16 -- one warp per row (consecutive lanes, consecutive bytes), grid-stride over rows.
+// status (may be null): the bytes of row i are zeroed where status_i != 0, by mask.
+__global__ void __launch_bounds__(256) k_copy_bytes(int n, int row_bytes, const uint8_t *__restrict__ src, size_t src_stride,
+                                                    uint8_t *__restrict__ dst, size_t dst_stride, const int *__restrict__ status) {
+    const int lane = threadIdx.x & 31;
+    for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
+        const uint8_t m = status ? (uint8_t)(0u - (uint32_t)(status[i] == 0)) : (uint8_t)0xFF;
+        const uint8_t *s = src + src_stride * i;
+        uint8_t *d = dst + dst_stride * i;
+        for (int b = lane; b < row_bytes; b += 32) d[b] = s[b] & m;
+    }
+}
+
+// The SecP256r1MLKEM768 outputs of item i from the dense images of its two halves, one warp per item, grid-stride:
+//   status_i = st_ec_i when it is -7 (the caller's own scalar), else st_mod_i when that is nonzero (st_mod may be null), else
+//   st_ec_i (-8 for the peer's point, or 0): the order of the checks is scalar, ek modulus, point;
+//   ss_i = ecdh_i || K_i, and (share != null) share_i[65, 1153) = c_i while share_i[0, 65) -- the P-256 public key k_p256 wrote
+//   there -- is kept; all zero where status_i != 0.  The status selects by mask, not by branch.
+__global__ void __launch_bounds__(256) k_p256_join(int n, const int *__restrict__ st_ec, const int *__restrict__ st_mod, int *__restrict__ status,
+                                                   const uint8_t *__restrict__ ecdh, const uint8_t *__restrict__ K, uint8_t *__restrict__ ss,
+                                                   const uint8_t *__restrict__ c, uint8_t *__restrict__ share) {
+    const int lane = threadIdx.x & 31;
+    for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
+        const int se = st_ec[i], sm = st_mod ? st_mod[i] : 0;
+        const int own = -(int)(se == -7);
+        const int s = (se & own) | (~own & (sm | (se & -(int)(sm == 0))));
+        const uint32_t m = 0u - (uint32_t)(s == 0);
+        if (lane < 4) {
+            uint4 v = lane < 2 ? reinterpret_cast<const uint4 *>(ecdh + 32 * (size_t)i)[lane] : reinterpret_cast<const uint4 *>(K + 32 * (size_t)i)[lane - 2];
+            reinterpret_cast<uint4 *>(ss + (size_t)kSecpSecret * i)[lane] = make_uint4(v.x & m, v.y & m, v.z & m, v.w & m);
+            if (lane == 0) status[i] = s;
+        }
+        if (share) {
+            uint8_t *row = share + (size_t)kSecpServerShare * i;
+            const uint8_t *crow = c + 1088 * (size_t)i;
+            for (int b = lane; b < kSecpServerShare; b += 32) row[b] = (b < kP256Point ? row[b] : crow[b - kP256Point]) & (uint8_t)m;
+        }
     }
 }
 

@@ -72,6 +72,13 @@ SIGNATURES = {
     "mlkem_b200_x25519mlkem768_decaps_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, C.c_void_p, _PO]),
     "mlkem_b200_x25519mlkem768_keygen_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _PO]),
     "mlkem_b200_x25519mlkem768_encaps_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_p256_public_batch": (C.c_int, [C.c_size_t, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_p256_ecdh_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_secp256r1mlkem768_keygen_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_secp256r1mlkem768_encaps_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_secp256r1mlkem768_decaps_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, C.c_void_p, _PO]),
+    "mlkem_b200_secp256r1mlkem768_keygen_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _PO]),
+    "mlkem_b200_secp256r1mlkem768_encaps_seeded_batch": (C.c_int, [C.c_size_t, _P8, _P8, _P8, _P8, C.c_void_p, _PO]),
     "mlkem_b200_pke_keygen_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _P8, _PO]),
     "mlkem_b200_pke_encrypt_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, _P8, _P8, _P8, _PO]),
     "mlkem_b200_pke_decrypt_batch": (C.c_int, [C.c_int, C.c_size_t, _P8, C.c_size_t, _P8, _P8, _PO]),

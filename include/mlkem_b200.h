@@ -329,6 +329,67 @@ int mlkem_b200_x25519mlkem768_encaps_seeded_batch(size_t n, const uint8_t *clien
                                                   uint8_t *server_share, uint8_t *ss, int32_t *status,
                                                   const mlkem_b200_opts *opts);
 
+/* ---- P-256 ECDH (FIPS 186-5, SP 800-56A) and the SecP256r1MLKEM768 hybrid key exchange (draft-ietf-tls-ecdhe-mlkem, TLS group
+ * 0x11EB) ---------------------------------------------------------------------------------------------------------------------- */
+
+/* Encodings: scalars are 32 bytes big-endian; points are the TLS 1.3 UncompressedPointRepresentation (RFC 8446 section
+ * 4.2.8.2), 0x04 || X || Y with 32-byte big-endian coordinates; the ECDH shared secret is the X coordinate of d Q, 32 bytes.
+ * Wire formats of SecP256r1MLKEM768, the P-256 part FIRST (unlike X25519MLKEM768; the draft's rule for the P-curve groups):
+ *   client share   P-256 public key (65)    || ML-KEM-768 ek (1184)
+ *   server share   P-256 public key (65)    || ML-KEM-768 ciphertext (1088)
+ *   shared secret  ECDH shared secret (32)  || ML-KEM shared secret (32)
+ *   client secret  ML-KEM-768 dk (2400)     || P-256 private scalar (32)      (library-defined, never on the wire)
+ * The 65 / 1249 / 1153-byte rows are not 16-byte multiples: a chunk_items the caller sets is rounded up to a multiple of 16. */
+#define MLKEM_B200_P256_POINT_BYTES 65
+#define MLKEM_B200_SECP256R1MLKEM768_CLIENT_SHARE_BYTES 1249
+#define MLKEM_B200_SECP256R1MLKEM768_CLIENT_SECRET_BYTES 2432
+#define MLKEM_B200_SECP256R1MLKEM768_SERVER_SHARE_BYTES 1153
+#define MLKEM_B200_SECP256R1MLKEM768_SHARED_SECRET_BYTES 64
+#define MLKEM_B200_ERR_EC_SCALAR (-7) /* per-item status: a P-256 private scalar outside [1, n - 1] */
+#define MLKEM_B200_ERR_EC_POINT (-8)  /* per-item status: a peer point fails SP 800-56A partial public-key validation */
+
+/* Every P-256 call reports per item, in status (n x int32 in opts->mem like the other buffers, not NULL: MLKEM_B200_ERR_ARG),
+ * and a failed item's outputs are all zero.  Checks, the first failing one wins: the caller's own scalar outside [1, n - 1]
+ * (MLKEM_B200_ERR_EC_SCALAR), then (hybrid encaps) the FIPS 203 modulus check of the ek part (MLKEM_B200_ERR_MODULUS), then
+ * the peer's point (MLKEM_B200_ERR_EC_POINT): first byte not 0x04, X >= p, Y >= p, or not on the curve.  With cofactor 1 that
+ * is all SP 800-56A asks of a peer key.  Every item is computed the same way whatever its status; only the outputs are masked.
+ * Constant-flow on the device: no branch, trip count or memory index depends on a scalar or a point (a 256-step Montgomery
+ * ladder over complete projective formulas). */
+/* scalar: n x 32.  pub: n x 65 = scalar G.  status: 0 or -7. */
+int mlkem_b200_p256_public_batch(size_t n, const uint8_t *scalar, uint8_t *pub, int32_t *status, const mlkem_b200_opts *opts);
+/* scalar: n x 32, peer: n x 65.  ss: n x 32 = X(scalar peer).  status: 0, -7 or -8. */
+int mlkem_b200_p256_ecdh_batch(size_t n, const uint8_t *scalar, const uint8_t *peer, uint8_t *ss, int32_t *status,
+                               const mlkem_b200_opts *opts);
+
+/* The three operations of SecP256r1MLKEM768.  ML-KEM always runs in FIPS 203 mode here, whatever opts->flags says;
+ * sample_group_limit, memory spaces, chunk_items, streams and MLKEM_B200_FLAG_ASYNC (host memory) behave as for the other
+ * calls.  Secrets: dk and the P-256 scalars exist only in the caller's buffers and in the chunk workspaces (wiped when freed). */
+/* d, z, ec_sk: n x 32.  client_share: n x 1249 = ec_sk G || ek.  client_secret: n x 2432 = dk || ec_sk.  (ek, dk) =
+ * ML-KEM.KeyGen_internal(d, z) in FIPS 203 mode.  status: 0 or -7 (client share and client secret zero). */
+int mlkem_b200_secp256r1mlkem768_keygen_batch(size_t n, const uint8_t *d, const uint8_t *z, const uint8_t *ec_sk,
+                                              uint8_t *client_share, uint8_t *client_secret, int32_t *status,
+                                              const mlkem_b200_opts *opts);
+/* client_share: n x 1249, m, ec_eph: n x 32.  server_share: n x 1153 = ec_eph G || c; ss: n x 64 = X(ec_eph client point) || K,
+ * (K, c) = ML-KEM.Encaps_internal(ek, m).  status: 0, -7, -4 or -8 (server share and ss zero). */
+int mlkem_b200_secp256r1mlkem768_encaps_batch(size_t n, const uint8_t *client_share, const uint8_t *m, const uint8_t *ec_eph,
+                                              uint8_t *server_share, uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts);
+/* client_secret: n x 2432, server_share: n x 1153.  ss: n x 64 = X(ec_sk server point) || ML-KEM.Decaps_internal(dk, c).
+ * status: 0, -7 (a stored scalar out of range) or -8; ML-KEM decapsulation never fails (a tampered ciphertext gives the
+ * implicit-rejection key). */
+int mlkem_b200_secp256r1mlkem768_decaps_batch(size_t n, const uint8_t *client_secret, const uint8_t *server_share,
+                                              uint8_t *ss, int32_t *status, const mlkem_b200_opts *opts);
+/* Randomness expanded on the device, as mlkem_b200_kem_*_seeded_batch (seed: HOST memory, 32 bytes or NULL = 32 bytes of
+ * /dev/urandom per call; synchronous in both memory spaces, MLKEM_B200_FLAG_ASYNC ignored; the seed is wiped):
+ *   keygen  (d_j, z_j) = R_j of tag 1 (exactly as mlkem_b200_kem_keygen_seeded_batch), ec_sk_j from R_j of tag 5;
+ *   encaps  m_j = R_j[0..32) of tag 2 (exactly as mlkem_b200_kem_encaps_seeded_batch), ec_eph_j from R_j of tag 6;
+ * where a scalar is (c mod (n - 1)) + 1 for c = the big-endian integer of R_j[0..40) (FIPS 186-5 A.2.1), always in range.
+ * No expanded secret crosses PCIe towards the device. */
+int mlkem_b200_secp256r1mlkem768_keygen_seeded_batch(size_t n, const uint8_t *seed, uint8_t *client_share,
+                                                     uint8_t *client_secret, const mlkem_b200_opts *opts);
+int mlkem_b200_secp256r1mlkem768_encaps_seeded_batch(size_t n, const uint8_t *client_share, const uint8_t *seed,
+                                                     uint8_t *server_share, uint8_t *ss, int32_t *status,
+                                                     const mlkem_b200_opts *opts);
+
 /* ---- K-PKE (FIPS 203 Alg. 13-15) -------------------------------------------------------------------- */
 
 /* PKE_KeyGen, ml_kem.c:651.  d: n x 32.  ek: n x (384k+32).  dk_pke: n x 384k. */
